@@ -69,7 +69,50 @@ def parse():
                     help="huber_delta of the ba_windows workload: 1.0 = the value the reference's demo tests with "
                          "(test_jac_Rt_gen.cpp:16), 1e-5 = the value jac_Rt_gen_.cpp:17 ships")
     ap.add_argument("--no-configs", action="store_true", help="skip the extra call-shape measurements (`configs`)")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the last timed step computed (rank 0) as DIR/<name>.npy "
+                         "(float64), so that two builds can be compared output for output on identical inputs")
+    a = ap.parse_args()
+    if a.dump_outputs and a.impl == "reference":
+        ap.error("--dump-outputs applies to the GPU arm (--impl ours)")
+    return a
+
+
+DUMP_MAX_ROWS = 32768           # pairs or windows dumped in full; beyond that a seeded sample (<= 42 MB either way)
+DUMP_DETAIL_BYTES = 16 << 20    # matches and masks (5 x kp float64 per pair) of a seeded sample of up to 32 pairs;
+                                # none when one pair's would exceed it, so a dump stays under 64 MB
+
+
+def dump_rows(n, cap, rng):
+    return np.arange(n) if n <= cap else np.sort(rng.choice(n, cap, replace=False))
+
+
+def dump_arrays(out_dir, arrays):
+    os.makedirs(out_dir, exist_ok=True)
+    for name, v in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), np.asarray(v, dtype=np.float64))
+
+
+def dump_pairs(out_dir, pipe, P, kp):
+    """What a caller of the resident path receives after its last step: the per-pair results (epivo_seq_download),
+    one array per field, and the matches and masks (epivo_seq_get_matches / _masks) of a seeded sample of pairs,
+    padded with -1 to kp entries.  pair_index / detail_pair_index name the pairs dumped."""
+    res = pipe.download(0, P)
+    rng = np.random.default_rng(0)
+    rows = dump_rows(P, DUMP_MAX_ROWS, rng)
+    out = {"pair_index": rows}
+    out.update({f: res[f][rows] for f in res.dtype.names})
+    detail = dump_rows(P, min(32, DUMP_DETAIL_BYTES // (40 * kp)), rng)
+    cols = {k: np.full((len(detail), kp), -1.0) for k in ("match_query", "match_train", "match_distance",
+                                                          "essential_mask", "pose_mask")}
+    for j, i in enumerate(detail):
+        qi, ti, d = pipe.matches(int(i))
+        em, pm = pipe.masks(int(i))
+        for k, v in zip(cols, (qi, ti, d, em, pm)):
+            cols[k][j, :len(v)] = v
+    out["detail_pair_index"] = detail
+    out.update(cols)
+    dump_arrays(out_dir, out)
 
 
 def config_of(a, world):
@@ -257,7 +300,8 @@ def windows_measure(a, ctx, world, rank, local, dist, steps, warmup, windows=Non
         dist.barrier()
     return {"windows": windows, "B": B, "k_ms": k_ms, "wall_ms": wall_ms, "launches": int(launches),
             "mean_iters": float(its.mean()) if B else 0.0, "h2d": int(T0.nbytes + pr.nbytes + p_r.nbytes),
-            "d2h": int(T0.nbytes + B * 28), "data": data, "nz": nz, "reps": reps}
+            "d2h": int(T0.nbytes + B * 28), "data": data, "nz": nz, "reps": reps,
+            "outputs": {"T": T, "H_norm_r_norm_lambda": res, "iters": its}}
 
 
 def run_windows(a):
@@ -278,6 +322,9 @@ def run_windows(a):
     clocks = ClockSampler(local)
     m = windows_measure(a, ctx, world, rank, local, dist, a.steps, a.warmup)
     clk = clocks.stop()
+    if a.dump_outputs and rank == 0:
+        rows = dump_rows(m["B"], DUMP_MAX_ROWS, np.random.default_rng(0))
+        dump_arrays(a.dump_outputs, {"window_index": rows, **{k: v[rows] for k, v in m["outputs"].items()}})
     line = {"metric": "kitti_ba windows/sec (windowed Rt LM, n_zeta 10, 20 reps x 250 correspondences, 30 iterations, "
                       "huber_delta %g)" % a.huber,
             "value": a.windows / (m["k_ms"] * 1e-3), "unit": "windows/s", "n_gpus": world, "steps": a.steps, "warmup": a.warmup,
@@ -605,6 +652,8 @@ def main():
     # ---------------- headline: device-resident, then end to end with host buffers ------------------
     clocks = ClockSampler(local)
     ms_step, stages, launches = run.resident(prm, a.steps, a.warmup)
+    if a.dump_outputs and rank == 0:
+        dump_pairs(a.dump_outputs, run.pipe, P, kp)
     value = world * P / (ms_step * 1e-3)
     ms_e2e = run.end_to_end(prm, a.steps)
     e2e_value = world * P / (ms_e2e * 1e-3)

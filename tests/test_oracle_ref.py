@@ -3,8 +3,10 @@ the reference's OWN code: /root/reference/jac_Rt_gen_.cpp compiled unmodified in
 (oracle/Makefile, oracle/ref_lm_tu.cpp, Eigen/Sophus stand-ins in oracle/ref_shim/), and against
 tests/golden/lm_ref.npz, the outputs of that build committed as fixtures
 (tests/golden/make_golden_lm_ref.py).  The live-library tests skip where oracle/_ref is absent;
-the golden tests always run."""
+the golden tests, and the stand-in's SE3::exp compiled on its own, always run."""
+import ctypes as C
 import os
+import subprocess
 
 import numpy as np
 import pytest
@@ -87,14 +89,39 @@ def test_res_and_jacobian_equal_reference_functions():
     assert np.abs(Ja - O.rep_jacobian(mem, 2, 1, 3, pr[4], p_r[4], 1.0)).max() <= 1e-10 * np.abs(Ja).max()
 
 
-@needs_ref
-def test_se3_exp_equals_sophus_standin():
+def _standin_se3_exp(tmp_dir):
+    """SE3::exp of the Sophus stand-in the reference build links, compiled on its own (tests/cpp/se3_exp_standin.cpp)
+    with the flags oracle/Makefile gives the stand-in."""
+    root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+    shim = os.path.join(root, "oracle", "ref_shim")
+    so = os.path.join(str(tmp_dir), "se3_exp_standin.so")
+    p = subprocess.run(["g++", "-O2", "-fPIC", "-ffp-contract=off", "-DNDEBUG", "-I", shim, "-shared",
+                        os.path.join(root, "tests", "cpp", "se3_exp_standin.cpp"), os.path.join(shim, "standin_impl.cpp"),
+                        "-o", so], capture_output=True, text=True)
+    assert p.returncode == 0, p.stderr
+    fn = C.CDLL(so).standin_se3_exp
+    fn.restype, fn.argtypes = None, [C.c_void_p, C.c_void_p]
+
+    def se3_exp(a):
+        a = np.ascontiguousarray(a, dtype=np.float64)
+        T = np.zeros((4, 4))
+        fn(a.ctypes.data, T.ctypes.data)
+        return T
+    return se3_exp
+
+
+def test_se3_exp_equals_sophus_standin(tmp_path):
+    """The numpy restatement against the stand-in's SE3::exp, and against the reference build's export of it where
+    that build is present."""
     rng = np.random.default_rng(3)
-    lib = reflib.ref()
+    impls = [_standin_se3_exp(tmp_path)]
+    if reflib.available() or os.path.exists(reflib.REFERENCE_SRC):
+        impls.append(reflib.ref().se3_exp)
     for scale in (1.0, 1e-3, 1e-8, 1e-12, 0.0):
         for _ in range(5):
             a = rng.normal(size=6) * np.array([1, 1, 1, scale, scale, scale])
-            assert np.abs(lib.se3_exp(a) - O.se3_exp(a)).max() < 1e-14
+            for se3_exp in impls:
+                assert np.abs(se3_exp(a) - O.se3_exp(a)).max() < 1e-14
 
 
 @needs_ref
