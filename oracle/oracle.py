@@ -97,19 +97,52 @@ def ratio_match(q, t, ratio=0.8, norm=NORM_HAMMING):
 # E1/E2: findEssentialMat                       kitti.cpp:98-104, kitti_E.cpp:98-104
 # ======================================================================================
 
+def _two_sum(a, b):
+    """Knuth's TwoSum: s = RN(a + b) and the exact error e = a + b - s."""
+    s = a + b
+    bb = s - a
+    return s, (a - (s - bb)) + (b - bb)
+
+
+def fma_f32_scalar(p: np.ndarray, a: float, b: float) -> np.ndarray:
+    """RN(p * a + b) with a single rounding (a fused multiply-add), elementwise, for float64 arrays p whose
+    values are float32-representable and float64 scalars a, b (no underflow / overflow).
+
+    Boldo & Melquiond, "Emulation of FMA and correctly rounded sums: proved algorithms using rounding to
+    odd" (IEEE TC 2008): with uh + ul = p a exactly and th + tl = b + uh exactly, RN(th + RO(tl + ul)) is
+    RN(p a + b).  p a is exact as two products: a = a1 + a2 with a1 the top 29 significant bits of a, so
+    p a1 (24 x 29 bits) and p a2 (24 x 24 bits) are both exact doubles."""
+    p = np.asarray(p, dtype=np.float64)
+    a1 = float((np.array([a], dtype=np.float64).view(np.int64) & ~np.int64((1 << 24) - 1)).view(np.float64)[0])
+    a2 = a - a1
+    uh, ul = _two_sum(p * a1, p * a2)
+    th, tl = _two_sum(np.full_like(p, b), uh)
+    v, e = _two_sum(tl, ul)
+    # round to odd: where v is inexact and its significand is even, step one ulp towards the exact sum
+    even = (v.view(np.int64) & 1) == 0
+    fix = (e != 0) & even
+    v = np.where(fix, np.nextafter(v, np.where(e > 0, np.inf, -np.inf)), v)
+    return th + v
+
+
 def normalize_points(p: np.ndarray, K: np.ndarray) -> np.ndarray:
     """five-point.cpp findEssentialMat: `points.col(0) = (points.col(0) - cx) / fx`.
 
     The MatExpr is folded by OpenCV into one scale-and-shift `u * (1/fx) + (-cx * (1/fx))`
-    (MatOp_AddEx::multiply), evaluated in float64 on the float32 pixels.
+    (MatOp_AddEx::multiply) and assigned with `convertTo(col, CV_64F, 1/fx, -cx/fx)`, evaluated in
+    float64 on the float32 pixels.  The per-element step of that conversion is FUSED: one rounding of
+    `u * (1/fx) + (-cx/fx)`.  Pinned against cv2 4.13.0 (x86-64; its dispatched conversion code is built
+    with FMA) by tests/test_oracle_sampson_boundary.py: a strided CV_64F column through `cv2.normalize`'s
+    NORM_MINMAX conversion, which is the same `convertTo(alpha, beta)` loop, matches the fused result on
+    every pixel where fused and un-fused differ (about half of them with the KITTI K).
     """
     p = np.asarray(p, dtype=np.float32).astype(np.float64).reshape(-1, 2)
     K = np.asarray(K, dtype=np.float64)
     ax, ay = 1.0 / K[0, 0], 1.0 / K[1, 1]
     bx, by = -K[0, 2] * ax, -K[1, 2] * ay
     out = np.empty_like(p)
-    out[:, 0] = p[:, 0] * ax + bx
-    out[:, 1] = p[:, 1] * ay + by
+    out[:, 0] = fma_f32_scalar(p[:, 0], ax, bx)
+    out[:, 1] = fma_f32_scalar(p[:, 1], ay, by)
     return out
 
 
@@ -383,6 +416,8 @@ def five_point(x1: np.ndarray, x2: np.ndarray, refine: bool = True) -> np.ndarra
             continue
         z = r.real
         Bz = _eval_B(B, z)[0]
+        if not np.isfinite(Bz).all():                # degenerate sample (no parallax): no model from this root
+            continue
         xy1 = np.linalg.svd(Bz)[2][2]
         if abs(xy1[2]) < 1e-10:
             continue
