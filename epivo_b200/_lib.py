@@ -92,6 +92,8 @@ SIGNATURES = {
     "epivo_orb_level_geometry": (_i, [_i, _i, _i, C.c_float, _i, _vp, _vp, _vp]),
     "epivo_remap": (_i, [_vp, _vp, _i, _i, _i, _vp, _vp, _i, _i, _i, _vp]),
     "epivo_seq_process_points": (_i, [_vp, C.POINTER(PipelineParams), _i, _vp, _vp, _vp, _i, _vp]),
+    "epivo_seq_process_frames": (_i, [_vp, C.POINTER(PipelineParams), _i, _vp, _i, _i, _vp, _vp, _i, _i, _i, _vp, _vp]),
+    "epivo_seq_get_points": (_i, [_vp, _i, _vp, _vp, _pi]),
     "epivo_microbench": (_i, [_vp, _i, C.POINTER(_d)]),
 }
 

@@ -568,6 +568,39 @@ class SequencePipeline:
         self.ctx.check(self.ctx.lib.epivo_seq_process_points(self.h, C.byref(params), n, _p(p0), _p(p1), _p(counts), cap, _p(out)))
         return out
 
+    def process_frames(self, params: PipelineParams, images, fastThreshold: int = 40, maps=None, corners: bool = False):
+        """The optical-flow loop body of kitti_E.cpp:54-201 / euroc_E.cpp:169-208 from frames, without leaving the device:
+        images (n, rows, cols) uint8 -> [remap with maps = (map_xy (h, w, 2) int16, map_frac (h, w) uint16)] -> FAST
+        (fastThreshold, non-maximum suppression) -> 21 x 21 pyramidal LK into the pair's second frame -> the tracks with
+        status 1 -> findEssentialMat -> recoverPose -> fallbacks -> LM, for the consecutive pairs or the pair list.
+        Returns the per-pair results, and with corners=True also the corners FAST found per frame."""
+        im = np.ascontiguousarray(images, dtype=np.uint8)
+        if im.ndim != 3:
+            raise ValueError("images must be (n, rows, cols) uint8")
+        n, rows, cols = im.shape
+        m1 = m2 = None
+        drows = dcols = 0
+        if maps is not None:
+            m1 = np.ascontiguousarray(maps[0], dtype=np.int16)
+            m2 = np.ascontiguousarray(maps[1], dtype=np.uint16)
+            if m1.ndim != 3 or m1.shape[2] != 2 or m2.shape != m1.shape[:2]:
+                raise ValueError("maps: (map_xy (h, w, 2) int16, map_frac (h, w) uint16)")
+            drows, dcols = m2.shape
+        n_out = self.n_pairs if self._pair_list else n - 1
+        out = np.zeros(max(n_out, 1), dtype=RESULT_DTYPE)
+        cnt = np.zeros(max(n, 1), dtype=np.int32)
+        self.ctx.check(self.ctx.lib.epivo_seq_process_frames(self.h, C.byref(params), n, _p(im), rows, cols, _p(m1), _p(m2),
+                                                              drows, dcols, int(fastThreshold), _p(cnt), _p(out)))
+        return (out[:n_out], cnt[:n]) if corners else out[:n_out]
+
+    def points(self, pair: int):
+        """After process_frames: the kept tracks of one pair in pixels -> (p0 (k, 2), p1 (k, 2)) float32."""
+        p0 = np.zeros((self.kp, 2), dtype=np.float32)
+        p1 = np.zeros((self.kp, 2), dtype=np.float32)
+        n = C.c_int(0)
+        self.ctx.check(self.ctx.lib.epivo_seq_get_points(self.h, int(pair), _p(p0), _p(p1), C.byref(n)))
+        return p0[:n.value], p1[:n.value]
+
     def download(self, first_pair: int, n_pairs: int, out=None):
         if out is None:
             out = np.zeros(n_pairs, dtype=RESULT_DTYPE)

@@ -379,11 +379,15 @@ __global__ void __launch_bounds__(128, EPV_LK_MINBLOCKS) lk_kernel(const uint8_t
                                                  const float* __restrict__ pts, const int32_t* __restrict__ counts,
                                                  int max_pts, int max_count, double eps2, float min_eig,
                                                  float* __restrict__ next_pts, uint8_t* __restrict__ status,
-                                                 float* __restrict__ err) {
+                                                 float* __restrict__ err, const int32_t* __restrict__ pair_frames) {
     const int pair = blockIdx.y, lane = threadIdx.x & 31;
     const int p = blockIdx.x * 4 + (threadIdx.x >> 5);
-    if (p >= counts[pair]) return;
-    const float px = pts[((size_t)pair * max_pts + p) * 2], py = pts[((size_t)pair * max_pts + p) * 2 + 1];
+    // pair i tracks frame i into frame i + 1 with the points and count of slot i; with pair_frames (gridDim.y pairs:
+    // previous frames, then next frames) it tracks the points of frame fi -- slot fi of pts / counts -- into frame fj
+    const int fi = pair_frames ? pair_frames[pair] : pair;
+    const int fj = pair_frames ? pair_frames[gridDim.y + pair] : pair + 1;
+    if (p >= min(counts[fi], max_pts)) return;
+    const float px = pts[((size_t)fi * max_pts + p) * 2], py = pts[((size_t)fi * max_pts + p) * 2 + 1];
     const float half = (LK_WIN - 1) * 0.5f;
     const float FLT_SCALE = 1.f / (1 << 20);
     float nx = 0.f, ny = 0.f;            // nextPts[ptidx]
@@ -394,9 +398,9 @@ __global__ void __launch_bounds__(128, EPV_LK_MINBLOCKS) lk_kernel(const uint8_t
     const int wyB = (lane + 32) / 3, wxB = LK_SEG * (lane + 32 - 3 * wyB);
     for (int level = g.levels - 1; level >= 0; --level) {
         const int rows = g.rows[level], cols = g.cols[level];
-        const uint8_t* I = pyr + (size_t)pair * g.frame_stride + g.off[level];
-        const uint8_t* J = pyr + (size_t)(pair + 1) * g.frame_stride + g.off[level];
-        const short2* dI = dpyr + (size_t)pair * g.frame_stride + g.off[level];
+        const uint8_t* I = pyr + (size_t)fi * g.frame_stride + g.off[level];
+        const uint8_t* J = pyr + (size_t)fj * g.frame_stride + g.off[level];
+        const short2* dI = dpyr + (size_t)fi * g.frame_stride + g.off[level];
         const float sc = 1.f / (float)(1 << level);
         float ppx = __fmul_rn(px, sc), ppy = __fmul_rn(py, sc);
         if (level == g.levels - 1) { nx = ppx; ny = ppy; } else { nx = __fmul_rn(nx, 2.f); ny = __fmul_rn(ny, 2.f); }
@@ -519,11 +523,10 @@ size_t epv_lk_work_bytes(int n_frames, int rows, int cols, int max_level) {
     return (size_t)n_frames * g.frame_stride * (1 + 4) + 1024;
 }
 
-// d_images: [n_frames][rows][cols]; pair i tracks d_pts[i][0..counts[i]) from frame i into frame i + 1
-int epv_lk_launch(epivo_ctx* ctx, const uint8_t* d_images, int n_frames, int rows, int cols, const float* d_pts,
-                  const int32_t* d_counts, int max_pts, int max_level, int max_count, double epsilon, double min_eig,
-                  float* d_next, uint8_t* d_status, float* d_err, void* work) {
-    if (n_frames < 2 || max_pts <= 0) return EPIVO_OK;
+// d_images: [n_frames][rows][cols] -> the pyramids of every frame in `work`, and the derivative pyramids of frames
+// [0, n_deriv) (the frames that are the previous image of some pair)
+int epv_lk_pyramids(epivo_ctx* ctx, const uint8_t* d_images, int n_frames, int rows, int cols, int max_level, int n_deriv,
+                    void* work) {
     if (rows <= LK_WIN || cols <= LK_WIN)
         EPV_FAIL(ctx, EPIVO_ERR_UNSUPPORTED, "image %d x %d not larger than the %d x %d window", cols, rows, LK_WIN, LK_WIN);
     if (n_frames > 65535) EPV_FAIL(ctx, EPIVO_ERR_UNSUPPORTED, "more than 65535 frames per call");
@@ -538,15 +541,43 @@ int epv_lk_launch(epivo_ctx* ctx, const uint8_t* d_images, int n_frames, int row
         pyr_down_kernel<<<dim3((n + 255) / 256, n_frames), 256, 0, ctx->stream>>>(pyr, g, l);
         EPV_LAUNCHED(ctx);
     }
-    for (int l = 0; l < g.levels; ++l) {                 // derivatives of the PREVIOUS image of every pair: frames 0 .. n-2
+    for (int l = 0; l < g.levels && n_deriv > 0; ++l) {
         const int n = g.rows[l] * g.cols[l];
-        scharr_kernel<<<dim3((n + 255) / 256, n_frames - 1), 256, 0, ctx->stream>>>(pyr, dpyr, g, l);
+        scharr_kernel<<<dim3((n + 255) / 256, n_deriv), 256, 0, ctx->stream>>>(pyr, dpyr, g, l);
         EPV_LAUNCHED(ctx);
     }
-    lk_kernel<<<dim3((max_pts + 3) / 4, n_frames - 1), 128, 0, ctx->stream>>>(pyr, dpyr, g, d_pts, d_counts, max_pts, max_count,
-                                                                            epsilon * epsilon, (float)min_eig, d_next, d_status, d_err);
+    return EPIVO_OK;
+}
+
+// LK over the pyramids epv_lk_pyramids left in `work` (built for n_frames frames): pair i < n_pairs tracks
+// d_pts[i][0..min(d_counts[i], max_pts)) from frame i into frame i + 1, or, with d_pair_frames (2 x n_pairs: previous
+// frames, then next frames), d_pts[fi][..d_counts[fi]) from frame fi = d_pair_frames[i] into d_pair_frames[n_pairs + i].
+// Outputs are [n_pairs][max_pts].
+int epv_lk_track_launch(epivo_ctx* ctx, const void* work, int n_frames, int rows, int cols, int max_level, int n_pairs,
+                        const int32_t* d_pair_frames, const float* d_pts, const int32_t* d_counts, int max_pts, int max_count,
+                        double epsilon, double min_eig, float* d_next, uint8_t* d_status, float* d_err) {
+    if (n_pairs <= 0 || max_pts <= 0) return EPIVO_OK;
+    if (n_pairs > 65535) EPV_FAIL(ctx, EPIVO_ERR_UNSUPPORTED, "more than 65535 pairs per call");
+    const LkGeom g = lk_geometry(rows, cols, max_level);
+    const uint8_t* pyr = (const uint8_t*)work;
+    const short2* dpyr = (const short2*)(pyr + (((size_t)n_frames * g.frame_stride + 255) & ~(size_t)255));
+    lk_kernel<<<dim3((max_pts + 3) / 4, n_pairs), 128, 0, ctx->stream>>>(pyr, dpyr, g, d_pts, d_counts, max_pts, max_count,
+                                                                       epsilon * epsilon, (float)min_eig, d_next, d_status,
+                                                                       d_err, d_pair_frames);
     EPV_LAUNCHED(ctx);
     return EPIVO_OK;
+}
+
+// d_images: [n_frames][rows][cols]; pair i tracks d_pts[i][0..counts[i]) from frame i into frame i + 1
+int epv_lk_launch(epivo_ctx* ctx, const uint8_t* d_images, int n_frames, int rows, int cols, const float* d_pts,
+                  const int32_t* d_counts, int max_pts, int max_level, int max_count, double epsilon, double min_eig,
+                  float* d_next, uint8_t* d_status, float* d_err, void* work) {
+    if (n_frames < 2 || max_pts <= 0) return EPIVO_OK;
+    // derivatives of the PREVIOUS image of every pair: frames 0 .. n-2
+    int rc = epv_lk_pyramids(ctx, d_images, n_frames, rows, cols, max_level, n_frames - 1, work);
+    if (rc) return rc;
+    return epv_lk_track_launch(ctx, work, n_frames, rows, cols, max_level, n_frames - 1, nullptr, d_pts, d_counts, max_pts,
+                               max_count, epsilon, min_eig, d_next, d_status, d_err);
 }
 
 // =================================================================================================================

@@ -37,6 +37,7 @@ struct epivo_seq {
     int max_pairs = 0, n_list = 0;   // capacity / pairs currently addressable
     int frames_hi = 0;               // frames [0, frames_hi) have been uploaded (plane pre-pass range in list mode)
     int list_max = 0;                // largest frame index the pair list references
+    std::vector<int32_t> h_fq, h_ft; // host copy of the pair list (epivo_seq_process_frames plans its windows from it)
     // per pair, whole sequence
     int32_t *d_mq = nullptr, *d_mt = nullptr, *d_md = nullptr, *d_nmatch = nullptr;
     uint8_t *d_emask = nullptr, *d_pmask = nullptr;
@@ -70,6 +71,10 @@ struct epivo_seq {
     int match_pad = 0;
     int last_mgroups = 0, last_ggroups = 0;
     int last_n_pairs = 0, last_first = 0;
+    // epivo_seq_process_frames: the kept tracks of every pair in pixels, [pair][p0 | p1][stride][2] floats (allocated by
+    // the first call); last_frames: the last run was process_frames, so epivo_seq_get_points may read them
+    float* d_trk = nullptr;
+    bool last_frames = false;
     std::vector<void*> allocs;
 };
 
@@ -140,6 +145,10 @@ __global__ void lm_prep_kernel(int n_pairs, int stride, epivo_pipeline_params pr
     }
 }
 
+// pixel -> K-normalised float64 coordinate, x = u / fx - cx / fx as the one fused scale-and-shift OpenCV's convertTo
+// computes (a = 1 / fx, b = -cx * a); every kernel that feeds the geometry with tracks calls this one function
+__device__ __forceinline__ double knorm(float u, double a, double b) { return __fma_rn((double)u, a, b); }
+
 // correspondences supplied by the caller (LK tracks, kitti_E.cpp:86-95) instead of descriptor matches: the same
 // pixel -> K-normalised float64 step the matcher's finalize kernel ends with, for a batch of pairs
 __global__ void __launch_bounds__(256) points_in_kernel(const float* __restrict__ p0, const float* __restrict__ p1,
@@ -154,12 +163,68 @@ __global__ void __launch_bounds__(256) points_in_kernel(const float* __restrict_
     const float2 a = reinterpret_cast<const float2*>(p0)[(size_t)pair * max_pts + i];
     const float2 b = reinterpret_cast<const float2*>(p1)[(size_t)pair * max_pts + i];
     double* x = xn + (size_t)pair * 4 * stride;
-    x[i] = __fma_rn((double)a.x, ax, bx);
-    x[stride + i] = __fma_rn((double)a.y, ay, by);
-    x[2 * stride + i] = __fma_rn((double)b.x, ax, bx);
-    x[3 * stride + i] = __fma_rn((double)b.y, ay, by);
+    x[i] = knorm(a.x, ax, bx);
+    x[stride + i] = knorm(a.y, ay, by);
+    x[2 * stride + i] = knorm(b.x, ax, bx);
+    x[3 * stride + i] = knorm(b.y, ay, by);
     mq[(size_t)pair * stride + i] = i;           // epivo_seq_get_matches then reports the identity association
     mt[(size_t)pair * stride + i] = i;
+}
+
+// kitti_E.cpp:86-95 on the device: one CTA per pair of a frame window keeps the LK tracks with status 1, in corner
+// order (ballot / popc offsets per warp, a running carry over the CTA), and writes them where the geometry reads
+// correspondences -- the same outputs as points_in_kernel on the filtered point lists.  meta: the window's pairs as
+// [previous frame][n], [next frame][n], [sequence pair index][n]; kps / found: the window's FAST corners and counts.
+__global__ void __launch_bounds__(256) track_compact_kernel(const int32_t* __restrict__ meta, int n, const float* __restrict__ kps,
+                                                            const int32_t* __restrict__ found, int kp,
+                                                            const float* __restrict__ next, const uint8_t* __restrict__ status,
+                                                            int stride, double ax, double bx, double ay, double by,
+                                                            float* __restrict__ trk, double* __restrict__ xn,
+                                                            int32_t* __restrict__ nmatch, int32_t* __restrict__ mq,
+                                                            int32_t* __restrict__ mt, int32_t* __restrict__ md) {
+    __shared__ int s_warp[8];
+    __shared__ int s_carry;
+    const int j = blockIdx.x, tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
+    const int fq = meta[j], pair = meta[2 * n + j];
+    const int cnt = min(found[fq], kp);
+    const float2* c = reinterpret_cast<const float2*>(kps) + (size_t)fq * kp;
+    const float2* nx = reinterpret_cast<const float2*>(next) + (size_t)j * kp;
+    const uint8_t* st = status + (size_t)j * kp;
+    float2* t0 = reinterpret_cast<float2*>(trk) + (size_t)pair * 2 * stride;
+    float2* t1 = t0 + stride;
+    double* x = xn + (size_t)pair * 4 * stride;
+    const size_t mo = (size_t)pair * stride;
+    if (tid == 0) s_carry = 0;
+    __syncthreads();
+    for (int base = 0; base < cnt; base += 256) {
+        const int i = base + tid;
+        const bool keep = i < cnt && st[i] == 1;
+        const unsigned bal = __ballot_sync(0xFFFFFFFFu, keep);
+        if (lane == 0) s_warp[warp] = __popc(bal);
+        __syncthreads();
+        int off = s_carry, total = 0;
+        for (int w = 0; w < 8; ++w) {
+            off += w < warp ? s_warp[w] : 0;
+            total += s_warp[w];
+        }
+        if (keep) {
+            const int k = off + __popc(bal & ((1u << lane) - 1));
+            const float2 a = c[i], b = nx[i];
+            t0[k] = a;
+            t1[k] = b;
+            x[k] = knorm(a.x, ax, bx);
+            x[stride + k] = knorm(a.y, ay, by);
+            x[2 * stride + k] = knorm(b.x, ax, bx);
+            x[3 * stride + k] = knorm(b.y, ay, by);
+            mq[mo + k] = i;                   // the track's corner in the query frame's FAST list
+            mt[mo + k] = i;
+            md[mo + k] = 0;
+        }
+        __syncthreads();
+        if (tid == 0) s_carry += total;
+        __syncthreads();
+    }
+    if (tid == 0) nmatch[pair] = s_carry;
 }
 
 __global__ void finish_kernel(int n_pairs, epivo_pipeline_params prm, const double* __restrict__ E,
@@ -378,6 +443,8 @@ int epivo_seq_set_pairs(epivo_seq* s, int n_pairs, const int32_t* fq, const int3
         s->list_max = lmax;                              // only once the whole list has been accepted
         s->pairs_set = true;
     }
+    s->h_fq.assign(h.begin(), h.begin() + n_pairs);
+    s->h_ft.assign(h.begin() + n_pairs, h.end());
     EPV_CUDA(ctx, cudaSetDevice(ctx->device));
     EPV_CUDA(ctx, cudaMemcpyAsync(s->d_fq, h.data(), (size_t)n_pairs * 4, cudaMemcpyHostToDevice, ctx->stream));
     EPV_CUDA(ctx, cudaMemcpyAsync(s->d_ft, h.data() + n_pairs, (size_t)n_pairs * 4, cudaMemcpyHostToDevice, ctx->stream));
@@ -726,6 +793,7 @@ static int seq_execute(epivo_seq* s, const epivo_pipeline_params* prm, int first
     if (n_m > HALF || n_g > HALF) EPV_FAIL(ctx, EPIVO_ERR_UNSUPPORTED, "too many pair groups");
     s->last_mgroups = n_m;
     s->last_ggroups = n_g;
+    s->last_frames = false;
     s->last_n_pairs = n_pairs;
     s->last_first = first_pair;
     // Host-buffer path: the geometry of the pairs already matched CAN run between the matcher pieces (four groups, own
@@ -899,6 +967,7 @@ int epivo_seq_process_points(epivo_seq* s, const epivo_pipeline_params* prm, int
     s->last_ggroups = n_g;
     s->last_n_pairs = n_pairs;
     s->last_first = 0;
+    s->last_frames = false;
     for (int c = 0; c < n_g; ++c) {
         const int g0 = c * SEQ_CHUNK, gn = std::min(SEQ_CHUNK, n_pairs - g0);
         rc = seq_run_geometry(s, prm, HALF + c, g0, gn);
@@ -906,6 +975,179 @@ int epivo_seq_process_points(epivo_seq* s, const epivo_pipeline_params* prm, int
     }
     EPV_CUDA(ctx, cudaEventRecord(s->ev_end, st));
     return epivo_seq_download(s, out, 0, n_pairs);
+}
+
+// The optical-flow loop body from frames (kitti_E.cpp:54-201, kitti.cpp, euroc_E.cpp:169-208).  The frames go through
+// the front end in windows of at most G frames, so that the workspace stays bounded on long sequences: per window one
+// upload, [remap], FAST capped at kp_per_frame, the pyramids and Scharr derivatives of every frame of the window, LK for
+// the pairs of the window and the status compaction into the sequence's correspondence buffers.  Consecutive windows
+// share S = max |ft - fq| frames, so every pair lies inside a window; a pair is tracked in the first window that holds
+// both of its frames.  The geometry then runs over all pairs as in epivo_seq_process_points (not interleaved with the
+// front end: overlapping the geometry with other work measured slower, see epivo_seq_set_overlap).
+namespace {
+constexpr int FRAMES_MAX_WINDOW = 256;
+constexpr size_t FRAMES_WS_BUDGET = (size_t)3 << 29;        // 1.5 GiB of front-end workspace per window
+constexpr int LK_WINDOW = 21, LK_MAX_LEVEL = 3, LK_MAX_COUNT = 30;   // calcOpticalFlowPyrLK's defaults, which every
+constexpr double LK_EPSILON = 0.01, LK_MIN_EIG = 1e-4;              // reference call site uses
+
+struct FramesWs {
+    size_t src, img, maps, fast, lk, kps;
+    size_t total() const { return src + img + maps + fast + lk + kps; }
+};
+FramesWs frames_ws(int g, int rows, int cols, int R, int C, bool maps, int kp) {
+    FramesWs w;
+    w.src = maps ? epv_align((size_t)g * rows * cols) : 0;
+    w.img = epv_align((size_t)g * R * C);
+    w.maps = maps ? epv_align((size_t)R * C * 4) + epv_align((size_t)R * C * 2) : 0;
+    w.fast = epv_align(epv_fast_work_bytes(g, R, C));
+    w.lk = epv_align(epv_lk_work_bytes(g, R, C, LK_MAX_LEVEL));
+    w.kps = epv_align((size_t)g * kp * 8);
+    return w;
+}
+}  // namespace
+
+int epivo_seq_process_frames(epivo_seq* s, const epivo_pipeline_params* prm, int n_frames, const uint8_t* images, int rows,
+                             int cols, const int16_t* map_xy, const uint16_t* map_frac, int drows, int dcols,
+                             int fast_threshold, int32_t* corners_out, epivo_pair_result* out) {
+    if (!s || !prm) return EPIVO_ERR_INVALID;
+    epivo_ctx* ctx = s->ctx;
+    // every check before the first launch
+    if (!images || !out) EPV_FAIL(ctx, EPIVO_ERR_INVALID, "null buffer");
+    if (n_frames < 2 || n_frames > s->max_frames) EPV_FAIL(ctx, EPIVO_ERR_INVALID, "n_frames %d outside [2,%d]", n_frames, s->max_frames);
+    if (rows <= 0 || cols <= 0) EPV_FAIL(ctx, EPIVO_ERR_INVALID, "empty frames (%d x %d)", cols, rows);
+    const bool maps = map_xy != nullptr || map_frac != nullptr;
+    if (maps && (!map_xy || !map_frac || drows <= 0 || dcols <= 0))
+        EPV_FAIL(ctx, EPIVO_ERR_INVALID, "remap needs both maps and a positive size (%d x %d)", dcols, drows);
+    const int R = maps ? drows : rows, C = maps ? dcols : cols;
+    if (R <= LK_WINDOW || C <= LK_WINDOW)
+        EPV_FAIL(ctx, EPIVO_ERR_UNSUPPORTED, "image %d x %d not larger than the %d x %d LK window", C, R, LK_WINDOW, LK_WINDOW);
+    if (fast_threshold < 0 || fast_threshold > 255) EPV_FAIL(ctx, EPIVO_ERR_INVALID, "fast_threshold %d outside [0, 255]", fast_threshold);
+    if (prm->lm_points < 1 || prm->lm_points > 64) EPV_FAIL(ctx, EPIVO_ERR_UNSUPPORTED, "lm_points must be in [1,64]");
+    if (prm->method != EPIVO_RANSAC && prm->method != EPIVO_LMEDS) EPV_FAIL(ctx, EPIVO_ERR_INVALID, "method");
+    if (s->pairs_set && s->list_max >= n_frames)
+        EPV_FAIL(ctx, EPIVO_ERR_INVALID, "the pair list references frame %d but only %d frames are given", s->list_max, n_frames);
+    const int n_pairs = s->pairs_set ? s->n_list : n_frames - 1;
+    constexpr int HALF = SEQ_MAX_CHUNKS / 2;
+    const int n_g = (n_pairs + SEQ_CHUNK - 1) / SEQ_CHUNK;
+    if (n_g > HALF) EPV_FAIL(ctx, EPIVO_ERR_UNSUPPORTED, "too many pair groups");
+    const int kp = s->kp, st = s->stride;
+    // window size G: at most 256 frames, and no more than the workspace budget holds
+    int G = std::min(FRAMES_MAX_WINDOW, n_frames);
+    while (G > 2 && frames_ws(G, rows, cols, R, C, maps, kp).total() > FRAMES_WS_BUDGET) --G;
+    int S = 0;
+    for (int p = 0; p < n_pairs; ++p) S = std::max(S, std::abs(s->h_ft[p] - s->h_fq[p]));
+    if (S >= G)
+        EPV_FAIL(ctx, EPIVO_ERR_UNSUPPORTED, "a pair spans %d frames; the front end tracks in windows of %d frames", S, G);
+    const int step = G - S;
+    const int n_win = 1 + (n_frames > G ? (n_frames - G + step - 1) / step : 0);
+    // pairs by window (list order inside a window): meta block of window k at 3 * first[k]
+    std::vector<int> win(n_pairs), first(n_win + 1, 0);
+    for (int p = 0; p < n_pairs; ++p) {
+        const int hi = std::max(s->h_fq[p], s->h_ft[p]);
+        win[p] = hi < G ? 0 : (hi - G + 1 + step - 1) / step;
+        ++first[win[p] + 1];
+    }
+    int max_wp = 0;
+    for (int k = 0; k < n_win; ++k) {
+        max_wp = std::max(max_wp, first[k + 1]);
+        first[k + 1] += first[k];
+    }
+    if (max_wp > 65535) EPV_FAIL(ctx, EPIVO_ERR_UNSUPPORTED, "%d pairs in one frame window (at most 65535)", max_wp);
+    std::vector<int32_t> meta((size_t)3 * n_pairs);
+    {
+        std::vector<int> fill(first.begin(), first.end() - 1);
+        for (int p = 0; p < n_pairs; ++p) {
+            const int k = win[p], nk = first[k + 1] - first[k], j = fill[k]++ - first[k];
+            int32_t* m = meta.data() + (size_t)3 * first[k];
+            m[j] = s->h_fq[p] - k * step;             // window-local frames
+            m[nk + j] = s->h_ft[p] - k * step;
+            m[2 * nk + j] = p;
+        }
+    }
+    EPV_CUDA(ctx, cudaSetDevice(ctx->device));
+    if (!s->d_trk) {
+        const int rc = seq_alloc(s, &s->d_trk, (size_t)s->max_pairs * st * 4);
+        if (rc) return rc;
+    }
+    const FramesWs w = frames_ws(G, rows, cols, R, C, maps, kp);
+    const size_t np = (size_t)max_wp * kp;
+    int rc = epv_ws_reserve(ctx, w.total() + epv_align((size_t)n_frames * 4) + epv_align(meta.size() * 4 + 4) +
+                                     epv_align(np * 8) + epv_align(np) + epv_align(np * 4) + 4096);
+    if (rc) return rc;
+    uint8_t* d_src = maps ? epv_ws_take<uint8_t>(ctx, w.src) : nullptr;
+    uint8_t* d_img = epv_ws_take<uint8_t>(ctx, w.img);
+    int16_t* d_mxy = maps ? epv_ws_take<int16_t>(ctx, (size_t)R * C * 2) : nullptr;
+    uint16_t* d_mfr = maps ? epv_ws_take<uint16_t>(ctx, (size_t)R * C) : nullptr;
+    uint8_t* d_fast = epv_ws_take<uint8_t>(ctx, w.fast);
+    uint8_t* d_lk = epv_ws_take<uint8_t>(ctx, w.lk);
+    float* d_kps = epv_ws_take<float>(ctx, (size_t)G * kp * 2);
+    int32_t* d_found = epv_ws_take<int32_t>(ctx, n_frames);
+    int32_t* d_meta = epv_ws_take<int32_t>(ctx, meta.size() + 1);
+    float* d_next = epv_ws_take<float>(ctx, np * 2);
+    uint8_t* d_status = epv_ws_take<uint8_t>(ctx, np);
+    float* d_err = epv_ws_take<float>(ctx, np);       // passed as every reference call site does: it gates the status
+    cudaStream_t cs = ctx->stream;
+    EpvRange r_seq(ctx, "epivo_seq_process_frames");
+    EPV_CUDA(ctx, cudaEventRecord(s->ev_begin, cs));
+    if (maps) {
+        EPV_CUDA(ctx, cudaMemcpyAsync(d_mxy, map_xy, (size_t)R * C * 4, cudaMemcpyHostToDevice, cs));
+        EPV_CUDA(ctx, cudaMemcpyAsync(d_mfr, map_frac, (size_t)R * C * 2, cudaMemcpyHostToDevice, cs));
+    }
+    EPV_CUDA(ctx, cudaMemcpyAsync(d_meta, meta.data(), meta.size() * 4, cudaMemcpyHostToDevice, cs));
+    const double ax = 1.0 / prm->K[0], ay = 1.0 / prm->K[4];
+    const double bx = -prm->K[2] * ax, by = -prm->K[5] * ay;
+    for (int k = 0; k < n_win; ++k) {
+        const int f0 = k * step, g = std::min(G, n_frames - f0), nk = first[k + 1] - first[k];
+        const size_t fb = (size_t)rows * cols;
+        EPV_CUDA(ctx, cudaMemcpyAsync(maps ? d_src : d_img, images + (size_t)f0 * fb, (size_t)g * fb, cudaMemcpyHostToDevice, cs));
+        if (maps) {
+            rc = epv_remap_launch(ctx, d_src, g, rows, cols, d_mxy, d_mfr, R, C, 0, d_img);
+            if (rc) return rc;
+        }
+        // a frame shared with the previous window is detected again: the same corners, the same count
+        rc = epv_fast_launch(ctx, d_img, g, R, C, fast_threshold, 1, kp, d_kps, nullptr, d_found + f0, d_fast);
+        if (rc) return rc;
+        if (nk == 0) continue;
+        rc = epv_lk_pyramids(ctx, d_img, g, R, C, LK_MAX_LEVEL, g, d_lk);
+        if (rc) return rc;
+        const int32_t* m = d_meta + (size_t)3 * first[k];
+        rc = epv_lk_track_launch(ctx, d_lk, g, R, C, LK_MAX_LEVEL, nk, m, d_kps, d_found + f0, kp, LK_MAX_COUNT, LK_EPSILON,
+                                 LK_MIN_EIG, d_next, d_status, d_err);
+        if (rc) return rc;
+        track_compact_kernel<<<nk, 256, 0, cs>>>(m, nk, d_kps, d_found + f0, kp, d_next, d_status, st, ax, bx, ay, by,
+                                                 s->d_trk, s->d_xn, s->d_nmatch, s->d_mq, s->d_mt, s->d_md);
+        EPV_LAUNCHED(ctx);
+    }
+    s->last_mgroups = 0;
+    s->last_ggroups = n_g;
+    s->last_n_pairs = n_pairs;
+    s->last_first = 0;
+    s->last_frames = true;
+    for (int c = 0; c < n_g; ++c) {
+        const int g0 = c * SEQ_CHUNK, gn = std::min(SEQ_CHUNK, n_pairs - g0);
+        rc = seq_run_geometry(s, prm, HALF + c, g0, gn);
+        if (rc) return rc;
+    }
+    EPV_CUDA(ctx, cudaEventRecord(s->ev_end, cs));
+    if (corners_out) EPV_CUDA(ctx, cudaMemcpyAsync(corners_out, d_found, (size_t)n_frames * 4, cudaMemcpyDeviceToHost, cs));
+    return epivo_seq_download(s, out, 0, n_pairs);
+}
+
+int epivo_seq_get_points(epivo_seq* s, int pair, float* p0, float* p1, int* n_out) {
+    if (!s || !n_out) return EPIVO_ERR_INVALID;
+    epivo_ctx* ctx = s->ctx;
+    if (!s->last_frames) EPV_FAIL(ctx, EPIVO_ERR_INVALID, "the last run was not epivo_seq_process_frames");
+    if (pair < 0 || pair >= s->last_n_pairs) EPV_FAIL(ctx, EPIVO_ERR_INVALID, "pair %d outside [0,%d)", pair, s->last_n_pairs);
+    EPV_CUDA(ctx, cudaSetDevice(ctx->device));
+    int32_t n = 0;
+    const float* t = s->d_trk + (size_t)pair * 4 * s->stride;
+    EPV_CUDA(ctx, cudaMemcpyAsync(&n, s->d_nmatch + pair, 4, cudaMemcpyDeviceToHost, ctx->stream));
+    EPV_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
+    if (p0) EPV_CUDA(ctx, cudaMemcpyAsync(p0, t, (size_t)n * 8, cudaMemcpyDeviceToHost, ctx->stream));
+    if (p1) EPV_CUDA(ctx, cudaMemcpyAsync(p1, t + 2 * (size_t)s->stride, (size_t)n * 8, cudaMemcpyDeviceToHost, ctx->stream));
+    EPV_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
+    *n_out = n;
+    return EPIVO_OK;
 }
 
 int epivo_seq_download(epivo_seq* s, epivo_pair_result* out, int first_pair, int n_pairs) {

@@ -82,6 +82,12 @@ size_t epv_lk_work_bytes(int n_frames, int rows, int cols, int max_level);
 int epv_lk_launch(epivo_ctx* ctx, const uint8_t* d_images, int n_frames, int rows, int cols, const float* d_pts,
                   const int32_t* d_counts, int max_pts, int max_level, int max_count, double epsilon, double min_eig,
                   float* d_next, uint8_t* d_status, float* d_err /* nullable */, void* work);
+// the two halves of epv_lk_launch, for callers that track a pair list over a batch of frames
+int epv_lk_pyramids(epivo_ctx* ctx, const uint8_t* d_images, int n_frames, int rows, int cols, int max_level, int n_deriv,
+                    void* work);
+int epv_lk_track_launch(epivo_ctx* ctx, const void* work, int n_frames, int rows, int cols, int max_level, int n_pairs,
+                        const int32_t* d_pair_frames /* nullable */, const float* d_pts, const int32_t* d_counts, int max_pts,
+                        int max_count, double epsilon, double min_eig, float* d_next, uint8_t* d_status, float* d_err);
 int epv_remap_launch(epivo_ctx* ctx, const uint8_t* d_img, int n_images, int rows, int cols, const int16_t* d_map_xy,
                      const uint16_t* d_map_frac, int drows, int dcols, int border, uint8_t* d_out);
 

@@ -257,6 +257,25 @@ int epivo_seq_process(epivo_seq* seq, const epivo_pipeline_params* p, int n_fram
  * counts[i]); epivo_seq_get_masks / epivo_seq_cloud work on them as after epivo_seq_process. */
 int epivo_seq_process_points(epivo_seq* seq, const epivo_pipeline_params* p, int n_pairs, const float* p0, const float* p1,
                              const int32_t* counts, int max_pts, epivo_pair_result* out);
+/* The loop body of kitti_E.cpp:54-201 / kitti.cpp / euroc_E.cpp:169-208 from 8-bit frames, on the device:
+ * [remap] -> FastFeatureDetector(fast_threshold, nonmax) on the first frame of every pair -> calcOpticalFlowPyrLK
+ * (21x21, maxLevel 3, 30 iterations, eps 0.01, minEig 1e-4, err passed: the reference's defaults) into the second
+ * frame -> keep the tracks with status 1, in corner order -> findEssentialMat -> recoverPose -> fallbacks -> LM.
+ * Pairs: consecutive (p, p+1) or the list of epivo_seq_set_pairs.  map_xy/map_frac: NULL, or the fixed-point maps
+ * of epivo_remap (drows x dcols; BORDER_CONSTANT 0), applied to every frame first.  A frame with more than
+ * kp_per_frame corners tracks the first kp_per_frame (OpenCV's order).  corners_out (nullable, n_frames entries):
+ * corners FAST found per frame.  out: one epivo_pair_result per pair, n_matches = tracks kept.
+ * images: n_frames x rows x cols, dense.  The front end runs in windows of at most 256 frames that overlap by the
+ * largest |ft - fq| of the pair list; a list whose span does not fit a window returns EPIVO_ERR_UNSUPPORTED.
+ * Afterwards epivo_seq_get_masks and epivo_seq_cloud work as after epivo_seq_process_points, and
+ * epivo_seq_get_matches reports for every kept track the index of its corner in the query frame's FAST list
+ * (query_idx == train_idx, dist 0). */
+int epivo_seq_process_frames(epivo_seq* seq, const epivo_pipeline_params* p, int n_frames, const uint8_t* images,
+                             int rows, int cols, const int16_t* map_xy, const uint16_t* map_frac, int drows, int dcols,
+                             int fast_threshold, int32_t* corners_out, epivo_pair_result* out);
+/* after epivo_seq_process_frames: the kept tracks of one pair in pixels (the reference's _cpt0 / _cpt1_), n_out x 2
+ * floats each (capacity kp_per_frame); EPIVO_ERR_INVALID unless the last run was epivo_seq_process_frames */
+int epivo_seq_get_points(epivo_seq* seq, int pair, float* p0, float* p1, int* n_out);
 /* device -> host copy of the results of the last run and stream sync */
 int epivo_seq_download(epivo_seq* seq, epivo_pair_result* out, int first_pair, int n_pairs);
 /* Scheduling of the geometry (findEssentialMat + recoverPose + LM) relative to the matcher; results do not depend on it.
