@@ -467,6 +467,7 @@ class SequencePipeline:
         self.max_pairs = self.max_frames - 1 if max_pairs is None else int(max_pairs)
         self.n_pairs = self.max_frames - 1
         self._pair_list = False
+        self._frames = self.max_frames          # frames given to the last process / process_frames call
         h = C.c_void_p()
         self.ctx.check(self.ctx.lib.epivo_seq_create_pairs(self.ctx.h, C.byref(h), self.max_frames, self.kp,
                                                            self.max_pairs))
@@ -543,6 +544,7 @@ class SequencePipeline:
             out = np.zeros(n_out, dtype=RESULT_DTYPE)
         assert out.dtype == RESULT_DTYPE and out.shape[0] >= n_out
         self.ctx.check(self.ctx.lib.epivo_seq_process(self.h, C.byref(params), F, _p(kps), _p(descs), _p(out)))
+        self._frames = F
         return out
 
     def process_points(self, params: PipelineParams, points0, points1, out=None):
@@ -591,6 +593,7 @@ class SequencePipeline:
         cnt = np.zeros(max(n, 1), dtype=np.int32)
         self.ctx.check(self.ctx.lib.epivo_seq_process_frames(self.h, C.byref(params), n, _p(im), rows, cols, _p(m1), _p(m2),
                                                               drows, dcols, int(fastThreshold), _p(cnt), _p(out)))
+        self._frames = n
         return (out[:n_out], cnt[:n]) if corners else out[:n_out]
 
     def points(self, pair: int):
@@ -600,6 +603,39 @@ class SequencePipeline:
         n = C.c_int(0)
         self.ctx.check(self.ctx.lib.epivo_seq_get_points(self.h, int(pair), _p(p0), _p(p1), C.byref(n)))
         return p0[:n.value], p1[:n.value]
+
+    def bundle_adjust(self, window, stride: int, K, num_frames: int | None = None, huber_delta: float = 1e-5,
+                      chains: bool = False):
+        """kitti_ba.cpp:757-905 (mono) over the pairs of the last run (`process`, `run` or `process_frames` over a pair list
+        that holds every window pair, e.g. `ba.window_pairs`), without the per-pair downloads: the same result as
+        `ba.match_kp` followed by `ba.bundle_adjustment(..., stereo=False)`.  window: the (first, second) offsets; K: the
+        intrinsics (inverted as `ba.assemble` does); num_frames: default the frames of the last process / process_frames.
+        Returns (opt_T (num_frames, 4, 4), lm (B, 3) [H_norm, r_norm, lambda], reverted (B,) bool, starts), and with
+        chains=True also the LM's per-window chains (B, n_zeta, 4, 4) and iteration counts (B,)."""
+        win = [(int(a), int(b)) for a, b in window]
+        if not win:
+            raise ValueError("empty window")
+        F = self._frames if num_frames is None else int(num_frames)
+        first = np.array([a for a, _ in win], dtype=np.int32)
+        second = np.array([b for _, b in win], dtype=np.int32)
+        Kinv = np.ascontiguousarray(np.linalg.inv(np.asarray(K, dtype=np.float64)))
+        nz = max(max(a, b) for a, b in win) - min(min(a, b) for a, b in win)
+        cap = max(1, (F + int(stride) - 1) // max(int(stride), 1))
+        opt = np.zeros((max(F, 1), 16), dtype=np.float64)
+        win_T = np.zeros((cap, max(nz, 1), 16), dtype=np.float64)
+        lm = np.zeros((cap, 3), dtype=np.float64)
+        its = np.zeros(cap, dtype=np.int32)
+        rev = np.zeros(cap, dtype=np.uint8)
+        nw = C.c_int32(0)
+        self.ctx.check(self.ctx.lib.epivo_seq_bundle_adjust(self.h, len(win), _p(first), _p(second), int(stride), F, _p(Kinv),
+                                                            float(huber_delta), _p(opt), _p(win_T), _p(lm), _p(its),
+                                                            _p(rev), C.byref(nw)))
+        B = nw.value
+        starts = list(range(0, B * int(stride), int(stride)))
+        out = (opt[:F].reshape(F, 4, 4), lm[:B], rev[:B].astype(bool), starts)
+        if chains:
+            out += (win_T[:B].reshape(B, nz, 4, 4), its[:B])
+        return out
 
     def download(self, first_pair: int, n_pairs: int, out=None):
         if out is None:

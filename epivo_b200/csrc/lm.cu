@@ -972,13 +972,22 @@ size_t lm_smem_doubles(int nz, int nr, int D, int threads, int tp, int cl) {
            (size_t)lm_tile_cols(D) * lm_tile_stride(tp) + D + 3 * (size_t)threads;
 }
 
+// the shared-memory test of one CTA shape: a window of n_zeta zetas and n_rep reps must fit
 template <int THREADS, int TP, int CL = 1>
-int lm_launch_shape(epivo_ctx* ctx, LmArgs& a) {
-    a.smem_doubles = lm_smem_doubles(a.p.n_zeta, a.p.n_rep, a.D, THREADS, TP, CL);
-    const size_t bytes = a.smem_doubles * sizeof(double);
+int lm_shape_fits(epivo_ctx* ctx, int n_zeta, int n_rep) {
+    const size_t bytes = lm_smem_doubles(n_zeta, n_rep, 6 * n_zeta, THREADS, TP, CL) * sizeof(double);
     if (bytes > LM_SMEM_LIMIT)
         EPV_FAIL(ctx, EPIVO_ERR_UNSUPPORTED, "LM problem needs %zu bytes of shared memory (n_zeta=%d, n_rep=%d)", bytes,
-                 a.p.n_zeta, a.p.n_rep);
+                 n_zeta, n_rep);
+    return EPIVO_OK;
+}
+
+template <int THREADS, int TP, int CL = 1>
+int lm_launch_shape(epivo_ctx* ctx, LmArgs& a) {
+    const int rc = lm_shape_fits<THREADS, TP, CL>(ctx, a.p.n_zeta, a.p.n_rep);
+    if (rc) return rc;
+    a.smem_doubles = lm_smem_doubles(a.p.n_zeta, a.p.n_rep, a.D, THREADS, TP, CL);
+    const size_t bytes = a.smem_doubles * sizeof(double);
     EPV_CUDA(ctx, cudaFuncSetAttribute(lm_kernel<THREADS, TP, CL>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bytes));
     if (CL == 1) {
         lm_kernel<THREADS, TP, CL><<<a.p.B, THREADS, bytes, ctx->stream>>>(a);
@@ -1002,6 +1011,13 @@ int lm_launch_shape(epivo_ctx* ctx, LmArgs& a) {
 }
 
 }  // namespace
+
+int epv_lm_check_n32(epivo_ctx* ctx, int n_zeta, int n_rep) {
+    if (n_zeta < 1 || n_zeta > LM_MAX_ZETA)
+        EPV_FAIL(ctx, EPIVO_ERR_UNSUPPORTED, "n_zeta = %d outside [1, %d]", n_zeta, LM_MAX_ZETA);
+    if (n_rep < 1) EPV_FAIL(ctx, EPIVO_ERR_INVALID, "n_rep = %d", n_rep);
+    return lm_shape_fits<64, 32>(ctx, n_zeta, n_rep);
+}
 
 int epv_lm_launch(epivo_ctx* ctx, const LmPlan& p) {
     if (p.B <= 0) return EPIVO_OK;

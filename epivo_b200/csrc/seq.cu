@@ -9,6 +9,8 @@
 #include <string.h>
 
 #include <algorithm>
+#include <cmath>
+#include <unordered_map>
 #include <vector>
 
 #include "common.cuh"
@@ -75,6 +77,11 @@ struct epivo_seq {
     // the first call); last_frames: the last run was process_frames, so epivo_seq_get_points may read them
     float* d_trk = nullptr;
     bool last_frames = false;
+    // what the last run left on the device for the pairs [last_first, +last_n_pairs) of the current pair list:
+    // matches into the frame slots' keypoints (run / process), kept tracks in d_trk (process_frames), or caller points
+    // that were not kept (process_points).  epivo_seq_bundle_adjust reads pixels from the first two, through the frames
+    // of the pair list, so unlike last_frames this is reset by epivo_seq_set_pairs.
+    enum { RUN_NONE, RUN_DESC, RUN_POINTS, RUN_FRAMES } last_run = RUN_NONE;
     std::vector<void*> allocs;
 };
 
@@ -225,6 +232,114 @@ __global__ void __launch_bounds__(256) track_compact_kernel(const int32_t* __res
         __syncthreads();
     }
     if (tid == 0) nmatch[pair] = s_carry;
+}
+
+// ---- windowed bundle adjustment (epivo_seq_bundle_adjust) -------------------------------------------------------------
+constexpr int BA_MIN_PT = 32;     // kitti_ba.cpp:777: points per reprojection
+
+struct BaKinv { double k[9]; };   // cam_, the inverse intrinsics, row-major
+
+// one row of cam_ * Vector3d(u, v, 1) as Eigen evaluates it (and ba.normalize's h @ Kinv.T): two products, two sums
+__device__ __forceinline__ double ba_knorm_row(const double* k, double u, double v) {
+    return __dadd_rn(__dadd_rn(__dmul_rn(k[0], u), __dmul_rn(k[1], v)), k[2]);
+}
+
+// the pair has a recoverPose estimate and points (ba.match_kp; kitti_ba.cpp:741-744 otherwise)
+__device__ __forceinline__ bool ba_pair_used(const int32_t* nmatch, const int32_t* ninl, int p) {
+    return nmatch[p] >= 8 && ninl[p] > 0;
+}
+
+// ba.match_kp + ba.assemble on the device: one CTA per (rep j, window b) reads pair p = tab[b][j] of the last run.
+// Its reprojection points are the matches (kept tracks) that are E-inliers AND whose recoverPose mask entry -- indexed by
+// the inlier's ordinal -- is 255, in match order; the first 32 are K-normalised into pr / p_r[b][j].  A scan of 256 entries
+// at a time takes two ballot / popc prefixes (inlier ordinal, kept ordinal) with running carries, and stops once 32 are
+// kept.  Fewer than 32 kept (or a pair without points): weight 0 and all-ones rows (kitti_ba.cpp:819-824), decided after
+// the scan, so no row is ever half written.  The rep-0 CTA of a window also writes the window's initial chain from the
+// (j, j+1) pairs tab[B * n_rep + b * n_zeta + k] into T0 (kept for the revert rule) and T (the LM's in/out chain).
+// Pixels: trk != NULL -> the kept tracks of process_frames, else the keypoints of the matched frame slots.
+__global__ void __launch_bounds__(256) ba_assemble_kernel(const int32_t* __restrict__ tab, int n_rep, int n_zeta, int stride,
+                                                          int kp, BaKinv ki, const int32_t* __restrict__ nmatch,
+                                                          const int32_t* __restrict__ ninl, const uint8_t* __restrict__ emask,
+                                                          const uint8_t* __restrict__ pmask, const double* __restrict__ R,
+                                                          const double* __restrict__ t, const int32_t* __restrict__ fq,
+                                                          const int32_t* __restrict__ ft, const int32_t* __restrict__ mq,
+                                                          const int32_t* __restrict__ mt, const float* __restrict__ kps,
+                                                          const float* __restrict__ trk, double* __restrict__ T0,
+                                                          double* __restrict__ T, double* __restrict__ pr,
+                                                          double* __restrict__ p_r, double* __restrict__ w) {
+    __shared__ int s_warp[2][8];
+    __shared__ int s_inl, s_keep;
+    __shared__ double s_rows[BA_MIN_PT][6];
+    const int j = blockIdx.x, b = blockIdx.y, B = gridDim.y, tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
+    const unsigned below = (1u << lane) - 1u;
+    const int p = tab[(size_t)b * n_rep + j];
+    const bool used = ba_pair_used(nmatch, ninl, p);
+    const int nm = used ? nmatch[p] : 0, ni = used ? ninl[p] : 0;
+    const size_t o = (size_t)p * stride;
+    const float2* kq = reinterpret_cast<const float2*>(kps) + (size_t)fq[p] * kp;
+    const float2* kt = reinterpret_cast<const float2*>(kps) + (size_t)ft[p] * kp;
+    const float2* t0 = trk ? reinterpret_cast<const float2*>(trk) + (size_t)p * 2 * stride : nullptr;
+    if (tid == 0) { s_inl = 0; s_keep = 0; }
+    __syncthreads();
+    for (int base = 0; base < nm; base += 256) {
+        const int i = base + tid;
+        const bool inl = i < nm && emask[o + i] == 1;
+        const unsigned bi = __ballot_sync(0xFFFFFFFFu, inl);
+        if (lane == 0) s_warp[0][warp] = __popc(bi);
+        __syncthreads();
+        int oi = s_inl, ti = 0;
+        for (int v = 0; v < 8; ++v) {
+            oi += v < warp ? s_warp[0][v] : 0;
+            ti += s_warp[0][v];
+        }
+        const int ji = oi + __popc(bi & below);                 // the inlier's ordinal: its recoverPose mask entry
+        const bool keep = inl && ji < ni && pmask[o + ji] == 255;
+        const unsigned bk = __ballot_sync(0xFFFFFFFFu, keep);
+        if (lane == 0) s_warp[1][warp] = __popc(bk);
+        __syncthreads();
+        int ok = s_keep, tk = 0;
+        for (int v = 0; v < 8; ++v) {
+            ok += v < warp ? s_warp[1][v] : 0;
+            tk += s_warp[1][v];
+        }
+        const int k = ok + __popc(bk & below);
+        if (keep && k < BA_MIN_PT) {
+            const float2 a = t0 ? t0[i] : kq[mq[o + i]];
+            const float2 c = t0 ? t0[stride + i] : kt[mt[o + i]];
+            for (int r = 0; r < 3; ++r) {
+                s_rows[k][r] = ba_knorm_row(ki.k + 3 * r, (double)a.x, (double)a.y);
+                s_rows[k][3 + r] = ba_knorm_row(ki.k + 3 * r, (double)c.x, (double)c.y);
+            }
+        }
+        __syncthreads();
+        if (tid == 0) {
+            s_inl += ti;
+            s_keep += tk;
+        }
+        __syncthreads();
+        if (s_keep >= BA_MIN_PT) break;
+    }
+    const bool full = s_keep >= BA_MIN_PT;
+    const size_t ro = ((size_t)b * n_rep + j) * BA_MIN_PT * 3;
+    for (int e = tid; e < BA_MIN_PT * 3; e += 256) {
+        pr[ro + e] = full ? s_rows[e / 3][e % 3] : 1.0;
+        p_r[ro + e] = full ? s_rows[e / 3][3 + e % 3] : 1.0;
+    }
+    if (tid == 0) w[(size_t)b * n_rep + j] = full ? 1.0 : 0.0;
+    if (j != 0) return;
+    for (int e = tid; e < n_zeta * 16; e += 256) {
+        const int k = e >> 4, r = (e >> 2) & 3, c = e & 3;
+        const int q = tab[(size_t)B * n_rep + (size_t)b * n_zeta + k];
+        const bool uq = ba_pair_used(nmatch, ninl, q);
+        const double fb = r == 2 ? -0.9 : 0.1;                  // kitti_ba.cpp:741-744: R = I, t = (0.1, 0.1, -0.9)
+        double v;
+        if (r == 3) v = c == 3 ? 1.0 : 0.0;
+        else if (c == 3) v = uq ? t[(size_t)q * 3 + r] : fb;
+        else v = uq ? R[(size_t)q * 9 + r * 3 + c] : (r == c ? 1.0 : 0.0);
+        const size_t to = ((size_t)b * n_zeta + k) * 16 + (r * 4 + c);
+        T0[to] = v;
+        T[to] = v;
+    }
 }
 
 __global__ void finish_kernel(int n_pairs, epivo_pipeline_params prm, const double* __restrict__ E,
@@ -445,6 +560,7 @@ int epivo_seq_set_pairs(epivo_seq* s, int n_pairs, const int32_t* fq, const int3
     }
     s->h_fq.assign(h.begin(), h.begin() + n_pairs);
     s->h_ft.assign(h.begin() + n_pairs, h.end());
+    s->last_run = epivo_seq::RUN_NONE;                   // pair p of the last run is no longer pair p of the list
     EPV_CUDA(ctx, cudaSetDevice(ctx->device));
     EPV_CUDA(ctx, cudaMemcpyAsync(s->d_fq, h.data(), (size_t)n_pairs * 4, cudaMemcpyHostToDevice, ctx->stream));
     EPV_CUDA(ctx, cudaMemcpyAsync(s->d_ft, h.data() + n_pairs, (size_t)n_pairs * 4, cudaMemcpyHostToDevice, ctx->stream));
@@ -794,6 +910,7 @@ static int seq_execute(epivo_seq* s, const epivo_pipeline_params* prm, int first
     s->last_mgroups = n_m;
     s->last_ggroups = n_g;
     s->last_frames = false;
+    s->last_run = epivo_seq::RUN_DESC;
     s->last_n_pairs = n_pairs;
     s->last_first = first_pair;
     // Host-buffer path: the geometry of the pairs already matched CAN run between the matcher pieces (four groups, own
@@ -968,6 +1085,7 @@ int epivo_seq_process_points(epivo_seq* s, const epivo_pipeline_params* prm, int
     s->last_n_pairs = n_pairs;
     s->last_first = 0;
     s->last_frames = false;
+    s->last_run = epivo_seq::RUN_POINTS;
     for (int c = 0; c < n_g; ++c) {
         const int g0 = c * SEQ_CHUNK, gn = std::min(SEQ_CHUNK, n_pairs - g0);
         rc = seq_run_geometry(s, prm, HALF + c, g0, gn);
@@ -1123,6 +1241,7 @@ int epivo_seq_process_frames(epivo_seq* s, const epivo_pipeline_params* prm, int
     s->last_n_pairs = n_pairs;
     s->last_first = 0;
     s->last_frames = true;
+    s->last_run = epivo_seq::RUN_FRAMES;
     for (int c = 0; c < n_g; ++c) {
         const int g0 = c * SEQ_CHUNK, gn = std::min(SEQ_CHUNK, n_pairs - g0);
         rc = seq_run_geometry(s, prm, HALF + c, g0, gn);
@@ -1282,6 +1401,171 @@ int epivo_seq_get_masks(epivo_seq* s, int pair, uint8_t* e_mask, int* n_e, uint8
     EPV_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
     if (n_e) *n_e = nm;
     if (n_pose) *n_pose = ni;
+    return EPIVO_OK;
+}
+
+// kitti_ba.cpp:757-905 (bundle_adjustment, mono) over the pairs of the last run: ba.match_kp + ba.bundle_adjustment
+// without the per-pair downloads.  Host: window plan and (frame, frame) -> pair lookup, every refusal before the first
+// launch.  Device: ba_assemble_kernel (one launch) -> the batched window LM (epv_lm_launch, as epivo_lm_rt_batch calls
+// it).  Host again: the sequential tail of ba.finish on the downloaded chains, O(windows x n_zeta).
+int epivo_seq_bundle_adjust(epivo_seq* s, int n_rep, const int32_t* first, const int32_t* second, int stride,
+                            int num_frames, const double Kinv[9], double huber_delta, double* opt_T, double* win_T,
+                            epivo_lm_res* lm, int32_t* iters, uint8_t* reverted, int32_t* n_windows) {
+    if (!s) return EPIVO_ERR_INVALID;
+    epivo_ctx* ctx = s->ctx;
+    if (!first || !second || !Kinv || !opt_T || !n_windows) EPV_FAIL(ctx, EPIVO_ERR_INVALID, "null argument");
+    if (n_rep < 1) EPV_FAIL(ctx, EPIVO_ERR_INVALID, "n_rep = %d: the window needs at least one pair", n_rep);
+    if (stride < 1) EPV_FAIL(ctx, EPIVO_ERR_INVALID, "stride = %d < 1", stride);
+    if (num_frames < 2 || num_frames > s->max_frames)
+        EPV_FAIL(ctx, EPIVO_ERR_INVALID, "num_frames %d outside [2,%d]", num_frames, s->max_frames);
+    if (s->last_run == epivo_seq::RUN_NONE)
+        EPV_FAIL(ctx, EPIVO_ERR_INVALID, "no run over the current pair list (epivo_seq_run / _process / _process_frames)");
+    if (s->last_run == epivo_seq::RUN_POINTS)
+        EPV_FAIL(ctx, EPIVO_ERR_INVALID, "the last run was epivo_seq_process_points, which keeps no pixels");
+    // window offsets -> reps and chain span (ba.window_reps, kitti_ba.cpp:810-815)
+    int lo = INT32_MAX, hi = 0;
+    std::vector<int32_t> reps((size_t)n_rep * 2);
+    for (int j = 0; j < n_rep; ++j) {
+        const int a = first[j], c = second[j];
+        if (a < 0 || c < 0) EPV_FAIL(ctx, EPIVO_ERR_INVALID, "window entry %d = (%d,%d) has a negative offset", j, a, c);
+        if (a == c) EPV_FAIL(ctx, EPIVO_ERR_INVALID, "window entry %d = (%d,%d) pairs a frame with itself", j, a, c);
+        reps[2 * j] = c > a ? a : a - 1;
+        reps[2 * j + 1] = c > a ? c - 1 : c;
+        lo = std::min(lo, std::min(a, c));
+        hi = std::max(hi, std::max(a, c));
+    }
+    const int n_zeta = hi - lo;
+    for (int j = 0; j < n_rep; ++j)      // ba.bundle_adjustment passes the reps unshifted: a window must start at offset 0
+        if (reps[2 * j] >= n_zeta || reps[2 * j + 1] >= n_zeta)
+            EPV_FAIL(ctx, EPIVO_ERR_INVALID, "rep %d = (%d,%d) outside the chain [0,%d)", j, reps[2 * j], reps[2 * j + 1], n_zeta);
+    int rc = epv_lm_check_n32(ctx, n_zeta, n_rep);
+    if (rc) return rc;
+    // window starts (ba.window_starts, kitti_ba.cpp:780-801): span = the largest offset
+    std::vector<int> starts;
+    for (int i = 0; i < num_frames; i += stride) {
+        if (i + hi >= num_frames) break;
+        starts.push_back(i);
+    }
+    const int B = (int)starts.size();
+    // (frame, frame) -> the first pair of the list with that key; every key must lie in the last run
+    std::unordered_map<int64_t, int> key;
+    key.reserve(s->h_fq.size() * 2);
+    for (size_t p = 0; p < s->h_fq.size(); ++p) key.emplace(((int64_t)s->h_fq[p] << 32) | (uint32_t)s->h_ft[p], (int)p);
+    std::vector<int32_t> tab((size_t)B * (n_rep + n_zeta));
+    auto lookup = [&](int b, int f0, int f1, int32_t* out) -> int {
+        const auto it = key.find(((int64_t)f0 << 32) | (uint32_t)f1);
+        if (it == key.end())
+            EPV_FAIL(ctx, EPIVO_ERR_INVALID, "window %d (start %d) needs the pair (%d,%d), which is not in the pair list", b,
+                     starts[b], f0, f1);
+        if (it->second < s->last_first || it->second >= s->last_first + s->last_n_pairs)
+            EPV_FAIL(ctx, EPIVO_ERR_INVALID, "the pair (%d,%d) is pair %d of the list, outside the last run [%d,+%d)", f0, f1,
+                     it->second, s->last_first, s->last_n_pairs);
+        *out = it->second;
+        return EPIVO_OK;
+    };
+    for (int b = 0; b < B && !rc; ++b) {
+        const int i = starts[b];
+        for (int j = 0; j < n_rep && !rc; ++j) rc = lookup(b, i + first[j], i + second[j], &tab[(size_t)b * n_rep + j]);
+        for (int k = 0; k < n_zeta && !rc; ++k)
+            rc = lookup(b, i + lo + k, i + lo + k + 1, &tab[(size_t)B * n_rep + (size_t)b * n_zeta + k]);
+    }
+    if (rc) return rc;
+    for (int f = 0; f < num_frames; ++f)
+        for (int e = 0; e < 16; ++e) opt_T[(size_t)f * 16 + e] = (e % 5 == 0) ? 1.0 : 0.0;
+    *n_windows = B;
+    if (B == 0) return EPIVO_OK;
+    // ---- device: assembly + LM
+    EPV_CUDA(ctx, cudaSetDevice(ctx->device));
+    EpvRange r_ba(ctx, "epivo_seq_bundle_adjust");
+    const size_t nT = (size_t)B * n_zeta * 16, nP = (size_t)B * n_rep * BA_MIN_PT * 3, nW = (size_t)B * n_rep;
+    const size_t n_tab = tab.size() + reps.size();
+    rc = epv_ws_reserve(ctx, epv_align(n_tab * 4) + 2 * epv_align(nT * 8) + 2 * epv_align(nP * 8) + epv_align(nW * 8) +
+                                 epv_align((size_t)B * sizeof(epivo_lm_res)) + epv_align((size_t)B * 4) + 4096);
+    if (rc) return rc;
+    rc = epv_pin_reserve(ctx, epv_align(n_tab * 4) + 2 * epv_align(nT * 8) + epv_align((size_t)B * sizeof(epivo_lm_res)) +
+                                  epv_align((size_t)B * 4) + 4096);
+    if (rc) return rc;
+    int32_t* d_tab = epv_ws_take<int32_t>(ctx, n_tab);
+    double* d_T0 = epv_ws_take<double>(ctx, nT);
+    double* d_T = epv_ws_take<double>(ctx, nT);
+    double* d_pr = epv_ws_take<double>(ctx, nP);
+    double* d_p_r = epv_ws_take<double>(ctx, nP);
+    double* d_w = epv_ws_take<double>(ctx, nW);
+    epivo_lm_res* d_lm = epv_ws_take<epivo_lm_res>(ctx, B);
+    int32_t* d_it = epv_ws_take<int32_t>(ctx, B);
+    int32_t* h_tab = epv_pin_take<int32_t>(ctx, n_tab);
+    double* h_T0 = epv_pin_take<double>(ctx, nT);
+    double* h_T = epv_pin_take<double>(ctx, nT);
+    epivo_lm_res* h_lm = epv_pin_take<epivo_lm_res>(ctx, B);
+    int32_t* h_it = epv_pin_take<int32_t>(ctx, B);
+    memcpy(h_tab, tab.data(), tab.size() * 4);
+    memcpy(h_tab + tab.size(), reps.data(), reps.size() * 4);
+    cudaStream_t st = ctx->stream;
+    EPV_CUDA(ctx, cudaMemcpyAsync(d_tab, h_tab, n_tab * 4, cudaMemcpyHostToDevice, st));
+    BaKinv ki;
+    memcpy(ki.k, Kinv, sizeof(ki.k));
+    const bool tracks = s->last_run == epivo_seq::RUN_FRAMES;
+    ba_assemble_kernel<<<dim3(n_rep, B), 256, 0, st>>>(d_tab, n_rep, n_zeta, s->stride, s->kp, ki, s->d_nmatch, s->d_ninl,
+                                                       s->d_emask, s->d_pmask, s->d_R, s->d_t, s->d_fq, s->d_ft, s->d_mq,
+                                                       s->d_mt, s->d_kps, tracks ? s->d_trk : nullptr, d_T0, d_T, d_pr,
+                                                       d_p_r, d_w);
+    EPV_LAUNCHED(ctx);
+    LmPlan lp{};
+    lp.B = B;
+    lp.n_zeta = n_zeta;
+    lp.n_rep = n_rep;
+    lp.N = BA_MIN_PT;
+    lp.reps = d_tab + tab.size();
+    lp.wreps = d_w;
+    lp.epsilon = 1e-8;                   // kitti_ba.cpp:881
+    lp.lambda0 = 1e-2;
+    lp.huber_delta = huber_delta;
+    lp.max_iters = 30;
+    lp.T0s = d_T;
+    lp.pr = d_pr;
+    lp.p_r = d_p_r;
+    lp.out = d_lm;
+    lp.iters = d_it;
+    lp.active = nullptr;
+    // the kernel choice of epivo_lm_rt_batch for the same reps, so both routes run the same code on the same bytes
+    lp.single_pair = (n_zeta == 1 && n_rep == 1 && reps[0] == 0 && reps[1] == 0) ? 1 : 0;
+    {
+        EpvRange r(ctx, "epivo: Levenberg_Marquardt (windows)");
+        rc = epv_lm_launch(ctx, lp);
+    }
+    if (rc) return rc;
+    EPV_CUDA(ctx, cudaMemcpyAsync(h_T0, d_T0, nT * 8, cudaMemcpyDeviceToHost, st));
+    EPV_CUDA(ctx, cudaMemcpyAsync(h_T, d_T, nT * 8, cudaMemcpyDeviceToHost, st));
+    EPV_CUDA(ctx, cudaMemcpyAsync(h_lm, d_lm, (size_t)B * sizeof(epivo_lm_res), cudaMemcpyDeviceToHost, st));
+    EPV_CUDA(ctx, cudaMemcpyAsync(h_it, d_it, (size_t)B * 4, cudaMemcpyDeviceToHost, st));
+    EPV_CUDA(ctx, cudaStreamSynchronize(st));
+    // ---- host: ba.finish (kitti_ba.cpp:853-856, 889-903).  A window whose r_norm exceeds 1e-2 keeps its initial chain
+    // (NaN does not revert, as in the reference's comparison); a window that starts on an optimized frame divides its
+    // translations by that frame's translation norm; later windows overwrite the overlap.
+    std::vector<uint8_t> optimized((size_t)num_frames, 0);
+    for (int b = 0; b < B; ++b) {
+        const int w0 = starts[b] + lo;
+        double scale = 1.0;
+        if (optimized[w0]) {
+            const double* tw = opt_T + (size_t)w0 * 16;
+            const double xx = tw[3] * tw[3], yy = tw[7] * tw[7], zz = tw[11] * tw[11];
+            scale = std::sqrt((xx + yy) + zz);
+        }
+        const bool rev = h_lm[b].r_norm > 1e-2;
+        const double* Ts = (rev ? h_T0 : h_T) + (size_t)b * n_zeta * 16;
+        for (int k = 0; k < n_zeta; ++k) {
+            double* o = opt_T + (size_t)(w0 + k) * 16;
+            memcpy(o, Ts + (size_t)k * 16, 128);
+            o[3] /= scale;
+            o[7] /= scale;
+            o[11] /= scale;
+            optimized[w0 + k] = 1;
+        }
+        if (reverted) reverted[b] = rev ? 1 : 0;
+    }
+    if (win_T) memcpy(win_T, h_T, nT * 8);
+    if (lm) memcpy(lm, h_lm, (size_t)B * sizeof(epivo_lm_res));
+    if (iters) memcpy(iters, h_it, (size_t)B * 4);
     return EPIVO_OK;
 }
 

@@ -296,6 +296,33 @@ int epivo_seq_get_matches(epivo_seq* seq, int pair, int32_t* query_idx, int32_t*
                           int32_t* dist, int* n_out);
 int epivo_seq_get_masks(epivo_seq* seq, int pair, uint8_t* e_mask, int* n_e, uint8_t* pose_mask, int* n_pose);
 
+/* ---- N3: windowed bundle adjustment over the pairs of the last run (mono) ----------------
+ * kitti_ba.cpp:757-905 (bundle_adjustment, mono) over the pairs of the last epivo_seq_run / epivo_seq_process /
+ * epivo_seq_process_frames, without leaving the device: the reprojections of match_kp (kitti_ba.cpp:583-755) are
+ * gathered from the pair data that run left, and every window's LM runs in one batched launch.
+ * window: n_rep offsets (first[j], second[j]) (kitti_ba.cpp:1131-1144, e.g. (0,1),(0,2),(1,2)); windows start at
+ * i = 0, stride, 2*stride, ... while i + max offset < num_frames (:780-801).  For window i, rep j uses the pair
+ * (i + first[j], i + second[j]) and the chain uses (i + lo + k, i + lo + k + 1), k < n_zeta = hi - lo (lo / hi: the
+ * smallest / largest offset).  All of these must be in the pair list -- a key listed twice means its first entry --
+ * and in the last run.  Per pair: fewer than 8 matches or no E-inlier -> R = I, t = (0.1, 0.1, -0.9) and no points
+ * (:741-744), else recoverPose's R, t and the matches (kept tracks) that are E-inliers with rec_mask == 255, in order;
+ * a rep gets its pair's first 32 such points, K-normalised as cam_ * (u, v, 1), or weight 0 with fewer (:819-824).
+ * LM: epsilon 1e-8, lambda0 1e-2, 30 iterations, N = 32 (:881).  Then the reference's sequential tail on the host:
+ * a window with r_norm > 1e-2 keeps its initial chain (:889-891), translations are divided by the norm of the
+ * translation of the window's first frame when an earlier window optimized it (:853-856, 898-901), later windows
+ * overwrite the overlap.  The result equals ba.match_kp followed by ba.bundle_adjustment(stereo=False).
+ * Kinv: the 3x3 inverse intrinsics, row-major (the driver's cam_).  opt_T: num_frames x 16 (identity where no window
+ * reaches).  win_T (n_zeta x 16 per window, the LM's chains before the revert rule) / lm / iters / reverted (nullable):
+ * per window, at most (num_frames + stride - 1) / stride entries; *n_windows: the number of windows.
+ * Refused before any launch: EPIVO_ERR_INVALID for a missing pair (named in the message), a pair outside the last run,
+ * first[j] == second[j], a negative offset, stride < 1, num_frames outside [2, max_frames], a last run of
+ * epivo_seq_process_points or no run over the current pair list; EPIVO_ERR_UNSUPPORTED for a window whose LM does not
+ * fit in shared memory (n_zeta > 18 or so).  No window fits: identity opt_T, *n_windows = 0, nothing launched.
+ * Stereo (bundle_adjustment_stereo) is not covered: its node layout and per-rep weights come from the driver. */
+int epivo_seq_bundle_adjust(epivo_seq* seq, int n_rep, const int32_t* first, const int32_t* second, int stride,
+                            int num_frames, const double Kinv[9], double huber_delta, double* opt_T, double* win_T,
+                            epivo_lm_res* lm, int32_t* iters, uint8_t* reverted, int32_t* n_windows);
+
 /* ---- N2: pose chain + depth / point cloud of the last run (kitti_E.cpp:203-254, euroc_E.cpp:303-349) ----
  * For the pairs [first_pair, +n_pairs) of the last epivo_seq_run / epivo_seq_process:
  *   dT_i     = [R_i | t_i/|t_i| * scales[i]]   (refined pose, GT-scaled translation; scales NULL = 1)
