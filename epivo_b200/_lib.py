@@ -95,6 +95,7 @@ SIGNATURES = {
     "epivo_seq_process_frames": (_i, [_vp, C.POINTER(PipelineParams), _i, _vp, _i, _i, _vp, _vp, _i, _i, _i, _vp, _vp]),
     "epivo_seq_get_points": (_i, [_vp, _i, _vp, _vp, _pi]),
     "epivo_seq_bundle_adjust": (_i, [_vp, _i, _vp, _vp, _i, _i, _vp, _d, _vp, _vp, _vp, _vp, _vp, _vp]),
+    "epivo_seq_bundle_adjust_stereo": (_i, [_vp, _i, _vp, _vp, _i, _i, _vp, _vp, _d, _vp, _vp, _vp, _vp, _vp, _vp]),
     "epivo_microbench": (_i, [_vp, _i, C.POINTER(_d)]),
 }
 

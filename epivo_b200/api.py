@@ -612,27 +612,55 @@ class SequencePipeline:
         intrinsics (inverted as `ba.assemble` does); num_frames: default the frames of the last process / process_frames.
         Returns (opt_T (num_frames, 4, 4), lm (B, 3) [H_norm, r_norm, lambda], reverted (B,) bool, starts), and with
         chains=True also the LM's per-window chains (B, n_zeta, 4, 4) and iteration counts (B,)."""
+        F = self._frames if num_frames is None else int(num_frames)
+        return self._bundle_adjust(False, window, stride, K, F, None, huber_delta, chains)
+
+    def bundle_adjust_stereo(self, window, stride: int, K, pair_weights=None, num_frames: int | None = None,
+                             huber_delta: float = 1e-5, chains: bool = False):
+        """kitti_ba.cpp:908-1068 (bundle_adjustment_stereo) over the pairs of the last run: the same result as `ba.match_kp`
+        with each reprojection's `w` set from pair_weights, followed by `ba.bundle_adjustment(..., stereo=True)`.  Frame f is
+        node 2f (left) and 2f + 1 (right), and the frame slots of the sequence are the nodes.  The pair list the call needs
+        is `ba.window_pairs(ba.expand_stereo_window(window), 2 * stride, 2 * num_frames)`.  window: the driver's frame
+        offsets, expanded as `ba.expand_stereo_window`; stride: in frames; pair_weights: one weight per pair of the current
+        list (the driver's reproj.w: 0 on the left -> right pairs (2f, 2f+1) freezes the rig extrinsics), None = 1.0;
+        num_frames: default half the frames of the last process / process_frames.  Returns (opt_T (2 * num_frames, 4, 4),
+        lm (B, 3), reverted (B,) bool, starts in frames), and with chains=True also the chains and iteration counts."""
+        F = self._frames // 2 if num_frames is None else int(num_frames)
+        pw = None
+        if pair_weights is not None:
+            pw = np.ascontiguousarray(pair_weights, dtype=np.float64).reshape(-1)
+            if pw.shape[0] != self.n_pairs:
+                raise ValueError(f"pair_weights has {pw.shape[0]} entries for {self.n_pairs} pairs")
+        return self._bundle_adjust(True, window, stride, K, F, pw, huber_delta, chains)
+
+    def _bundle_adjust(self, stereo, window, stride, K, F, pw, huber_delta, chains):
+        from .ba import expand_stereo_window
         win = [(int(a), int(b)) for a, b in window]
         if not win:
             raise ValueError("empty window")
-        F = self._frames if num_frames is None else int(num_frames)
         first = np.array([a for a, _ in win], dtype=np.int32)
         second = np.array([b for _, b in win], dtype=np.int32)
         Kinv = np.ascontiguousarray(np.linalg.inv(np.asarray(K, dtype=np.float64)))
-        nz = max(max(a, b) for a, b in win) - min(min(a, b) for a, b in win)
+        nodes = expand_stereo_window(win) if stereo else win
+        nz = max(max(a, b) for a, b in nodes) - min(min(a, b) for a, b in nodes)
+        n_opt = 2 * F if stereo else F
         cap = max(1, (F + int(stride) - 1) // max(int(stride), 1))
-        opt = np.zeros((max(F, 1), 16), dtype=np.float64)
+        opt = np.zeros((max(n_opt, 1), 16), dtype=np.float64)
         win_T = np.zeros((cap, max(nz, 1), 16), dtype=np.float64)
         lm = np.zeros((cap, 3), dtype=np.float64)
         its = np.zeros(cap, dtype=np.int32)
         rev = np.zeros(cap, dtype=np.uint8)
         nw = C.c_int32(0)
-        self.ctx.check(self.ctx.lib.epivo_seq_bundle_adjust(self.h, len(win), _p(first), _p(second), int(stride), F, _p(Kinv),
-                                                            float(huber_delta), _p(opt), _p(win_T), _p(lm), _p(its),
-                                                            _p(rev), C.byref(nw)))
+        tail = (_p(Kinv), float(huber_delta), _p(opt), _p(win_T), _p(lm), _p(its), _p(rev), C.byref(nw))
+        if stereo:
+            self.ctx.check(self.ctx.lib.epivo_seq_bundle_adjust_stereo(self.h, len(win), _p(first), _p(second), int(stride),
+                                                                       F, _p(pw), *tail))
+        else:
+            self.ctx.check(self.ctx.lib.epivo_seq_bundle_adjust(self.h, len(win), _p(first), _p(second), int(stride), F,
+                                                                *tail))
         B = nw.value
         starts = list(range(0, B * int(stride), int(stride)))
-        out = (opt[:F].reshape(F, 4, 4), lm[:B], rev[:B].astype(bool), starts)
+        out = (opt[:n_opt].reshape(n_opt, 4, 4), lm[:B], rev[:B].astype(bool), starts)
         if chains:
             out += (win_T[:B].reshape(B, nz, 4, 4), its[:B])
         return out

@@ -317,11 +317,36 @@ int epivo_seq_get_masks(epivo_seq* seq, int pair, uint8_t* e_mask, int* n_e, uin
  * Refused before any launch: EPIVO_ERR_INVALID for a missing pair (named in the message), a pair outside the last run,
  * first[j] == second[j], a negative offset, stride < 1, num_frames outside [2, max_frames], a last run of
  * epivo_seq_process_points or no run over the current pair list; EPIVO_ERR_UNSUPPORTED for a window whose LM does not
- * fit in shared memory (n_zeta > 18 or so).  No window fits: identity opt_T, *n_windows = 0, nothing launched.
- * Stereo (bundle_adjustment_stereo) is not covered: its node layout and per-rep weights come from the driver. */
+ * fit in shared memory (n_zeta > 18 or so).  No window fits: identity opt_T, *n_windows = 0, nothing launched. */
 int epivo_seq_bundle_adjust(epivo_seq* seq, int n_rep, const int32_t* first, const int32_t* second, int stride,
                             int num_frames, const double Kinv[9], double huber_delta, double* opt_T, double* win_T,
                             epivo_lm_res* lm, int32_t* iters, uint8_t* reverted, int32_t* n_windows);
+
+/* ---- N3: windowed bundle adjustment over the pairs of the last run (stereo) --------------
+ * kitti_ba.cpp:908-1068 (bundle_adjustment_stereo): epivo_seq_bundle_adjust with the stereo node layout.  Frame f of
+ * the rig is node 2f (left) and node 2f + 1 (right); the frame slots of the sequence are the nodes, so the last run
+ * covered 2 * num_frames slots.  window: the driver's n_rep frame offsets (first[j], second[j]), e.g. (0,1),(0,2),(1,2);
+ * each entry (a, b) becomes the three node reps (2a, 2b), (2a+1, 2b), (2a, 2a+1) (:934-941), so ws = 3 has 9 reps over
+ * n_zeta = 4 nodes.  stride is in frames: windows start at frame i = 0, stride, ... while 2i + the largest node offset
+ * < 2 * num_frames (:943-963), and use the node pairs (2i + a', 2i + b') of the expanded reps and the chain
+ * (2i + lo + k, 2i + lo + k + 1).  The pair list that holds every key the windows read, chain pairs (2f+1, 2f+2)
+ * included, is ba.window_pairs(ba.expand_stereo_window(window), 2 * stride, 2 * num_frames).
+ * pair_w (nullable): one weight per entry of the current pair list, indexed as epivo_seq_set_pairs -- the reproj.w of
+ * that pair; NULL is 1.0 everywhere.  The driver sets 0 on the left -> right pairs (2f, 2f+1) to freeze the rig
+ * extrinsics (:171-172, :1000-1008).  A rep with 32 points weighs its pair's pair_w and carries its real K-normalised
+ * rows even when that weight is 0; a rep with fewer weighs 0 with all-ones rows.  A key listed twice uses its first
+ * entry, for the points and the weight alike.  The selection, fallbacks, LM and revert rule are the mono call's; there is
+ * no scale carry (:1054-1066): later windows overwrite the overlap with their chains unscaled.  The result equals
+ * ba.match_kp with each reproj.w set from pair_w, followed by ba.bundle_adjustment(stereo=True).
+ * opt_T: 2 * num_frames x 16 (identity where no window reaches).  win_T / lm / iters / reverted / *n_windows as in the
+ * mono call.  Refused before any launch: everything the mono call refuses, with num_frames outside [2, max_frames / 2]
+ * and a window offset of max_frames / 2 or more; a non-finite pair_w entry (EPIVO_ERR_INVALID).  EPIVO_ERR_UNSUPPORTED
+ * when the expanded window's LM does not fit (n_zeta = 2 * the largest frame offset, in nodes).  No window fits:
+ * identity opt_T for the 2 * num_frames nodes, *n_windows = 0, nothing launched. */
+int epivo_seq_bundle_adjust_stereo(epivo_seq* seq, int n_rep, const int32_t* first, const int32_t* second, int stride,
+                                   int num_frames, const double* pair_w, const double Kinv[9], double huber_delta,
+                                   double* opt_T, double* win_T, epivo_lm_res* lm, int32_t* iters, uint8_t* reverted,
+                                   int32_t* n_windows);
 
 /* ---- N2: pose chain + depth / point cloud of the last run (kitti_E.cpp:203-254, euroc_E.cpp:303-349) ----
  * For the pairs [first_pair, +n_pairs) of the last epivo_seq_run / epivo_seq_process:

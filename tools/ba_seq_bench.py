@@ -1,13 +1,18 @@
-"""The mono windowed bundle adjustment of kitti_ba.cpp over a drive, two ways, alternating in one process (one JSON line):
+"""The windowed bundle adjustment of kitti_ba.cpp over a drive, two ways, alternating in one process (one JSON line):
   composed  ba.match_kp (set_pairs -> process -> per-pair downloads and a numpy selection) -> ba.bundle_adjustment
             (ba.assemble on the host, one epivo_lm_rt_batch, ba.finish)
-  resident  SequencePipeline: set_pairs -> process -> bundle_adjust (assembly and LM on the device, the tail on the host)
-Both routes create their own pipeline, as ba.match_kp does.  Workload: synth.make_sequence(1009 frames, 2000 keypoints),
-window {(0,1),(0,2),(1,2)}, stride 2 (1512 pairs, 504 windows), findEssentialMat(LMEDS, .99, .1).  Times are wall clock
-of whole calls (each ends in a stream synchronise); medians over the rounds after one warm-up round.  The outputs of the
-two routes are compared with test_gpu_ba's tolerances (rotation 1e-4 rad, translation direction 1e-3 rad, r_norm rtol
-1e-4, the same reverted windows).
-    python tools/ba_seq_bench.py [frames] [reps]"""
+  resident  SequencePipeline: set_pairs -> process -> bundle_adjust / bundle_adjust_stereo (assembly and LM on the device,
+            the tail on the host)
+Both routes create their own pipeline, as ba.match_kp does.  Workload: window {(0,1),(0,2),(1,2)}, stride 2,
+findEssentialMat(LMEDS, .99, .1), on
+  mono      synth.make_sequence(1009 frames, 2000 keypoints): 1512 pairs, 504 windows;
+  --stereo  synth.make_sequence(2 * 1009 nodes, 2000 keypoints), node 2f the left and 2f + 1 the right image of frame f:
+            the window expands to 9 node reps over 4 nodes, 4032 node pairs, 504 windows, and every left -> right pair
+            (2f, 2f+1) has weight 0 as the driver sets it (kitti_ba.cpp:1000-1008).
+Times are wall clock of whole calls (each ends in a stream synchronise); medians over the rounds after one warm-up round.
+The outputs of the two routes are compared with test_gpu_ba's tolerances (rotation 1e-4 rad, translation direction 1e-3
+rad, r_norm rtol 1e-4, the same reverted windows).
+    python tools/ba_seq_bench.py [--stereo] [frames] [reps]"""
 import json
 import os
 import subprocess
@@ -32,22 +37,36 @@ def device_info():
     return q
 
 
-def composed(ctx, seq, F):
+def rig_weight(a, b):
+    """The stereo driver's reproj.w: 0 on the left -> right pairs (2f, 2f+1), which freezes the rig extrinsics."""
+    return 0.0 if a % 2 == 0 and b == a + 1 else 1.0
+
+
+def composed(ctx, seq, F, stereo):
     t0 = time.perf_counter()
-    reprojs = ba.match_kp(seq.kps, seq.descs, WINDOW, STRIDE, seq.K, ctx=ctx)
+    if stereo:
+        reprojs = ba.match_kp(seq.kps, seq.descs, ba.expand_stereo_window(WINDOW), 2 * STRIDE, seq.K, ctx=ctx)
+        for (a, b), r in reprojs.items():
+            r.w = rig_weight(a, b)
+    else:
+        reprojs = ba.match_kp(seq.kps, seq.descs, WINDOW, STRIDE, seq.K, ctx=ctx)
     t1 = time.perf_counter()
-    out = ba.bundle_adjustment(reprojs, WINDOW, STRIDE, F, seq.K, False, 1e-5, ctx=ctx)
+    out = ba.bundle_adjustment(reprojs, WINDOW, STRIDE, F, seq.K, stereo, 1e-5, ctx=ctx)
     t2 = time.perf_counter()
     return out, {"total": t2 - t0, "match_kp": t1 - t0, "bundle_adjustment": t2 - t1}
 
 
-def resident(ctx, seq, F, pairs, prm):
+def resident(ctx, seq, pairs, prm, pair_w):
     t0 = time.perf_counter()
-    pipe = api.SequencePipeline(F, seq.kps.shape[1], ctx=ctx, max_pairs=max(len(pairs), F - 1))
+    n = seq.kps.shape[0]
+    pipe = api.SequencePipeline(n, seq.kps.shape[1], ctx=ctx, max_pairs=max(len(pairs), n - 1))
     pipe.set_pairs([p[0] for p in pairs], [p[1] for p in pairs])
     pipe.process(prm, seq.kps, seq.descs)
     t1 = time.perf_counter()
-    out = pipe.bundle_adjust(WINDOW, STRIDE, seq.K, huber_delta=1e-5)
+    if pair_w is None:
+        out = pipe.bundle_adjust(WINDOW, STRIDE, seq.K, huber_delta=1e-5)
+    else:
+        out = pipe.bundle_adjust_stereo(WINDOW, STRIDE, seq.K, pair_weights=pair_w, huber_delta=1e-5)
     t2 = time.perf_counter()
     pipe.close()
     return out, {"total": t2 - t0, "process": t1 - t0, "bundle_adjust": t2 - t1}
@@ -79,26 +98,38 @@ def agree(a, b):
 
 
 def main():
-    F = int(sys.argv[1]) if len(sys.argv) > 1 else 1009
-    reps = int(sys.argv[2]) if len(sys.argv) > 2 else 10
+    args = [a for a in sys.argv[1:] if a != "--stereo"]
+    stereo = len(args) < len(sys.argv) - 1
+    F = int(args[0]) if len(args) > 0 else 1009
+    reps = int(args[1]) if len(args) > 1 else 10
     os.environ.pop("EPIVO_LM_SHAPE", None)
-    seq = synth.make_sequence(n_frames=F, n=2000)
-    pairs = ba.window_pairs(WINDOW, STRIDE, F)
+    if stereo:
+        seq = synth.make_sequence(n_frames=2 * F, n=2000)
+        pairs = ba.window_pairs(ba.expand_stereo_window(WINDOW), 2 * STRIDE, 2 * F)
+        pair_w = np.array([rig_weight(a, b) for a, b in pairs])
+        workload = ("make_sequence(%d nodes = %d stereo frames, 2000), window %s expanded to %d node reps, stride %d "
+                    "frames, weight 0 on (2f, 2f+1): %d pairs, %%d windows, LMEDS(.99, .1)"
+                    % (2 * F, F, WINDOW, len(ba.expand_stereo_window(WINDOW)), STRIDE, len(pairs)))
+    else:
+        seq = synth.make_sequence(n_frames=F, n=2000)
+        pairs = ba.window_pairs(WINDOW, STRIDE, F)
+        pair_w = None
+        workload = ("make_sequence(%d, 2000), window %s, stride %d: %d pairs, %%d windows, LMEDS(.99, .1)"
+                    % (F, WINDOW, STRIDE, len(pairs)))
     prm = api.default_params(np.asarray(seq.K, dtype=np.float32), method=api.LMEDS, prob=0.99, threshold=0.1)
     ctx = api.Context(0)
     info = device_info()
     tc, tr, diffs = [], [], []
     for _ in range(reps + 1):                          # the first round is the warm-up
-        a, ta = composed(ctx, seq, F)
-        b, tb = resident(ctx, seq, F, pairs, prm)
+        a, ta = composed(ctx, seq, F, stereo)
+        b, tb = resident(ctx, seq, pairs, prm, pair_w)
         tc.append(ta)
         tr.append(tb)
         diffs.append(agree(b, a))
     tc, tr = tc[1:], tr[1:]
     med = lambda rows, k: float(np.median([r[k] for r in rows])) * 1e3          # noqa: E731
     out = {"device": info,
-           "workload": "make_sequence(%d, 2000), window %s, stride %d: %d pairs, %d windows, LMEDS(.99, .1)"
-                       % (F, WINDOW, STRIDE, len(pairs), len(b[3])),
+           "workload": workload % len(b[3]),
            "method": "wall clock of whole calls, median of %d alternating rounds after one warm-up round" % reps,
            "composed_ms_median": {k: med(tc, k) for k in tc[0]},
            "resident_ms_median": {k: med(tr, k) for k in tr[0]},
