@@ -80,7 +80,6 @@ SIGNATURES = {
     "epivo_seq_download": (_i, [_vp, _vp, _i, _i]),
     "epivo_seq_process": (_i, [_vp, C.POINTER(PipelineParams), _i, _vp, _vp, _vp]),
     "epivo_seq_stage_ms": (_i, [_vp, _vp, _i]),
-    "epivo_seq_set_overlap": (_i, [_vp, _i]),
     "epivo_seq_get_matches": (_i, [_vp, _i, _vp, _vp, _vp, _pi]),
     "epivo_seq_get_masks": (_i, [_vp, _i, _vp, _pi, _vp, _pi]),
     "epivo_seq_cloud": (_i, [_vp, _vp, _i, _i, _vp, _vp, C.c_int64, _vp, C.POINTER(C.c_int64)]),

@@ -672,12 +672,6 @@ class SequencePipeline:
         self.ctx.check(self.ctx.lib.epivo_seq_download(self.h, _p(out), int(first_pair), int(n_pairs)))
         return out
 
-    def set_overlap(self, on):
-        """Scheduling of the geometry relative to the matcher (epivo_seq_set_overlap): False / 0 = default (after the
-        matcher), True / 1 = two-stream pipelining across pair groups for resident data, 2 = the geometry between the
-        matcher pieces of the host-buffer path.  Results do not depend on it; both options measured slower."""
-        self.ctx.check(self.ctx.lib.epivo_seq_set_overlap(self.h, int(on)))
-
     def stage_ms(self):
         ms = np.zeros(16, dtype=np.float32)
         self.ctx.check(self.ctx.lib.epivo_seq_stage_ms(self.h, _p(ms), 16))

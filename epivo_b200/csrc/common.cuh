@@ -103,7 +103,6 @@ struct MatchPlan {
     uint32_t* colkey;          // [n_pairs][stride]
     int stride;
     cudaEvent_t ev0 = nullptr, ev1 = nullptr;   // optional: recorded right around the tile kernel
-    int pad_smem = 0;          // extra dynamic shared memory per CTA (bytes) to cap resident CTAs per SM
     // optional general addressing (device arrays; all three or none): pair p matches frame fq[p] against frame
     // ft[p] of a frame array with qs (= ts) rows per slot, counts[frame] of them valid; q0 / t0 are ignored
     const int32_t* fq = nullptr;

@@ -370,10 +370,7 @@ int launch_words(epivo_ctx* ctx, const MatchPlan& mp, const uint32_t* src) {
     const bool n2 = mp.norm == EPIVO_NORM_HAMMING2;
 #define EPV_MT(N2, T2, CN)                                                                                 \
     do {                                                                                                   \
-        if (mp.pad_smem > 0)                                                                               \
-            cudaFuncSetAttribute(match_tile_kernel<WORDS, RQ, N2, T2, CN>, cudaFuncAttributeMaxDynamicSharedMemorySize, \
-                                 mp.pad_smem);                                                             \
-        match_tile_kernel<WORDS, RQ, N2, T2, CN><<<grid, block, mp.pad_smem, ctx->stream>>>(               \
+        match_tile_kernel<WORDS, RQ, N2, T2, CN><<<grid, block, 0, ctx->stream>>>(                         \
             src, mp.q0, mp.qs, mp.t0, mp.ts, mp.nq, mp.nt, mp.rowkey, mp.rowkey2, mp.colkey, mp.stride, tps, part, \
             mp.fq, mp.ft, mp.counts);                                                                      \
     } while (0)

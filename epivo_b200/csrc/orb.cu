@@ -25,7 +25,7 @@
 namespace {
 
 constexpr int ORB_MAX_LEVELS = 16;
-constexpr int ORB_HALF_PATCH = 15;
+constexpr int ORB_PATCH_RADIUS = 15;
 constexpr int ORB_PATCH = 31;
 
 struct OrbGeom {
@@ -274,10 +274,10 @@ __global__ void __launch_bounds__(256) orb_describe_kernel(OrbGeom g, const uint
         // ICAngles: m_10 = sum u I(u, v), m_01 = sum v I(u, v) over the disc; lane = column u + 15
         int m10 = 0, m01 = 0;
         if (lane < ORB_PATCH) {
-            const int u = lane - ORB_HALF_PATCH, au = abs(u);
+            const int u = lane - ORB_PATCH_RADIUS, au = abs(u);
             const uint8_t* c = im + (size_t)y * cols + (x + u);
             int col = c[0];
-            for (int v = 1; v <= ORB_HALF_PATCH; ++v) {
+            for (int v = 1; v <= ORB_PATCH_RADIUS; ++v) {
                 if (au > c_umax[v]) break;                                // umax decreases with v
                 const int plus = c[(ptrdiff_t)v * cols], minus = c[-(ptrdiff_t)v * cols];
                 col += plus + minus;
@@ -362,8 +362,8 @@ int epv_orb_plan(epivo_ctx* ctx, int n_images, int rows, int cols, int nfeatures
                  int edge_threshold, int max_kp, EpvOrbPlan* plan) {
     if (nlevels < 1 || nlevels > ORB_MAX_LEVELS) EPV_FAIL(ctx, EPIVO_ERR_UNSUPPORTED, "nlevels %d outside [1, %d]", nlevels, ORB_MAX_LEVELS);
     if (!(scale_factor > 1.0f) || scale_factor > 2.0f) EPV_FAIL(ctx, EPIVO_ERR_UNSUPPORTED, "scale_factor %g outside (1, 2]", scale_factor);
-    if (edge_threshold < ORB_HALF_PATCH)       // the orientation disc must stay inside the level
-        EPV_FAIL(ctx, EPIVO_ERR_UNSUPPORTED, "edge_threshold %d below the patch radius %d", edge_threshold, ORB_HALF_PATCH);
+    if (edge_threshold < ORB_PATCH_RADIUS)       // the orientation disc must stay inside the level
+        EPV_FAIL(ctx, EPIVO_ERR_UNSUPPORTED, "edge_threshold %d below the patch radius %d", edge_threshold, ORB_PATCH_RADIUS);
     if (nfeatures < 0) EPV_FAIL(ctx, EPIVO_ERR_INVALID, "negative nfeatures");
     OrbGeom& g = *reinterpret_cast<OrbGeom*>(plan->geom);
     static_assert(sizeof(OrbGeom) <= sizeof(plan->geom), "EpvOrbPlan::geom too small");
@@ -408,7 +408,7 @@ int epivo_orb_level_geometry(int rows, int cols, int nfeatures, float scale_fact
     if (rows <= 0 || cols <= 0 || !level_rows || !level_cols || !level_features) return EPIVO_ERR_INVALID;
     epivo_ctx scratch;                         // host-only: carries the error text of epv_orb_plan, no CUDA call is made
     EpvOrbPlan plan;
-    const int rc = epv_orb_plan(&scratch, 1, rows, cols, nfeatures, scale_factor, nlevels, ORB_HALF_PATCH, 0, &plan);
+    const int rc = epv_orb_plan(&scratch, 1, rows, cols, nfeatures, scale_factor, nlevels, ORB_PATCH_RADIUS, 0, &plan);
     if (rc) return rc;
     const OrbGeom& g = *reinterpret_cast<const OrbGeom*>(plan.geom);
     for (int l = 0; l < nlevels; ++l) {

@@ -5,12 +5,12 @@
 // of kitti_ba.cpp:641-693 as the correspondence source.  Pairs are processed in chunks so
 // that a chunk's intermediates (keys, matches, normalised points, masks) stay L2-resident;
 // everything is enqueued on the context stream with no host synchronisation in between.
-#include <stdlib.h>
 #include <string.h>
 
 #include <algorithm>
 #include <cmath>
 #include <unordered_map>
+#include <utility>
 #include <vector>
 
 #include "common.cuh"
@@ -18,14 +18,14 @@
 
 namespace {
 constexpr int SEQ_CHUNK = 8192;          // pairs per launch group (single stream: large groups, fewer tails)
-constexpr int SEQ_CHUNK_OVERLAP = 1024;  // group size when the two-stream pipelining is switched on
-constexpr int SEQ_STAGES = 7;      // prep, match, finalize, essential, pose, lm, (total)
-constexpr int SEQ_MAX_CHUNKS = 256;
+constexpr int SEQ_MAX_GROUPS = 128;      // matcher groups (upload pieces) and geometry groups per run, each
+constexpr int SEQ_MATCH_EVENTS = 4;      // per matcher group: begin, end, tile kernel begin, tile kernel end
+constexpr int SEQ_GEO_EVENTS = 6;        // per geometry group: the five stage boundaries, then presolve done
 }  // namespace
 
 struct epivo_seq {
     epivo_ctx* ctx = nullptr;
-    int max_frames = 0, kp = 0, stride = 0, chunk = SEQ_CHUNK;
+    int max_frames = 0, kp = 0, stride = 0;
     // frames
     float* d_kps = nullptr;
     uint32_t* d_desc = nullptr;
@@ -57,20 +57,14 @@ struct epivo_seq {
     size_t esswork_bytes = 0;
     // host staging for results
     epivo_pair_result* h_results = nullptr;
-    // timing
-    cudaEvent_t ev[SEQ_MAX_CHUNKS][SEQ_STAGES] = {};
-    cudaEvent_t evk[SEQ_MAX_CHUNKS][2] = {};     // around the matcher tile kernel alone
-    cudaEvent_t evp[SEQ_MAX_CHUNKS] = {};        // after sample + presolve
+    // events (epivo_seq_stage_ms reads the timed ones)
+    cudaEvent_t ev_match[SEQ_MAX_GROUPS][SEQ_MATCH_EVENTS] = {};
+    cudaEvent_t ev_geo[SEQ_MAX_GROUPS][SEQ_GEO_EVENTS] = {};
+    cudaEvent_t ev_landed[SEQ_MAX_GROUPS] = {};  // host-buffer path, copy stream: the frames of matcher piece c are on the device
     cudaEvent_t ev_begin = nullptr, ev_end = nullptr;
-    cudaStream_t stream2 = nullptr;          // geometry stream (FP64 kernels) -- overlaps the integer-bound matcher
+    cudaEvent_t ev_join = nullptr;               // host-buffer path: stream3's matcher pieces, joined before the geometry
+    cudaStream_t stream2 = nullptr;          // host-buffer path: copy stream (uploads, HAMMING2 planes of each piece)
     cudaStream_t stream3 = nullptr;          // host-buffer path: every other matcher piece (see seq_execute)
-    cudaStream_t stream4 = nullptr;          // host-buffer path, copy-bound regime: geometry of the groups already matched
-    cudaEvent_t ev_piece[SEQ_MAX_CHUNKS] = {};   // matcher piece c (tiles + finalize) complete
-    int geo_mode = 0;                        // 2: geometry between the matcher pieces of the host-buffer path (epivo_seq_set_overlap)
-    cudaEvent_t ev_matched[SEQ_MAX_CHUNKS] = {};
-    cudaEvent_t ev_geo_done = nullptr;
-    int overlap = 0;   // measured on B200: co-running the matcher and the FP64 kernels gains nothing (see DESIGN.md)
-    int match_pad = 0;
     int last_mgroups = 0, last_ggroups = 0;
     int last_n_pairs = 0, last_first = 0;
     // epivo_seq_process_frames: the kept tracks of every pair in pixels, [pair][p0 | p1][stride][2] floats (allocated by
@@ -81,7 +75,7 @@ struct epivo_seq {
     // matches into the frame slots' keypoints (run / process), kept tracks in d_trk (process_frames), or caller points
     // that were not kept (process_points).  epivo_seq_bundle_adjust reads pixels from the first two, through the frames
     // of the pair list, so unlike last_frames this is reset by epivo_seq_set_pairs.
-    enum { RUN_NONE, RUN_DESC, RUN_POINTS, RUN_FRAMES } last_run = RUN_NONE;
+    enum RunKind { RUN_NONE, RUN_DESC, RUN_POINTS, RUN_FRAMES } last_run = RUN_NONE;
     std::vector<void*> allocs;
 };
 
@@ -95,6 +89,46 @@ int seq_alloc(epivo_seq* s, T** p, size_t count) {
     s->allocs.push_back(q);
     *p = reinterpret_cast<T*>(q);
     return EPIVO_OK;
+}
+
+// every event of a sequence object, array by array, with its creation flags (epivo_seq_create / _destroy)
+struct SeqEventArray {
+    cudaEvent_t* ev;
+    int n;
+    unsigned flags;
+};
+constexpr int SEQ_EVENT_ARRAYS = 6;
+void seq_event_arrays(epivo_seq* s, SeqEventArray (&a)[SEQ_EVENT_ARRAYS]) {
+    a[0] = {&s->ev_match[0][0], SEQ_MAX_GROUPS * SEQ_MATCH_EVENTS, cudaEventDefault};
+    a[1] = {&s->ev_geo[0][0], SEQ_MAX_GROUPS * SEQ_GEO_EVENTS, cudaEventDefault};
+    a[2] = {s->ev_landed, SEQ_MAX_GROUPS, cudaEventDisableTiming};
+    a[3] = {&s->ev_begin, 1, cudaEventDefault};
+    a[4] = {&s->ev_end, 1, cudaEventDefault};
+    a[5] = {&s->ev_join, 1, cudaEventDisableTiming};
+}
+
+// Upload pieces of the host-buffer path over pairs [first_pair, +n_pairs), as (first pair, pairs); wave: pairs per
+// full wave of matcher CTAs.  A quarter wave first (the matcher starts 0.1 ms after the call instead of 0.43), doubling
+// up to one wave: 74, 148, 296, 296, ... pairs (measured 17.17 -> 16.94 ms per step against 16.65 device-resident);
+// the last piece takes the rest when less than a quarter wave would be left.  Small pieces are what matters when the
+// copy is slower than the matcher: alone on a box the PCIe copy delivers frames 2x faster than the matcher consumes
+// them (55 GB/s against 26 GB/s) and any schedule hides it, but with eight ranks pulling at once a rank gets 23 GB/s
+// (profiles/r2_h2d_ceiling_8gpu.json), the matcher runs behind the copy, and the step ends one piece of matching after
+// the last byte lands (round 1's 1, 2, 4, rest schedule left 2468 pairs = 7.5 ms there).
+std::vector<std::pair<int, int> > seq_upload_pieces(int first_pair, int n_pairs, int wave) {
+    const int q = std::max(1, wave / 4);
+    int cap = 4;                                    // in quarter waves
+    // never more pieces than event slots: widen the cap for very long sequences
+    while ((n_pairs + (int64_t)q * cap - 1) / ((int64_t)q * cap) + 2 > SEQ_MAX_GROUPS && cap < (1 << 20)) cap *= 2;
+    std::vector<std::pair<int, int> > pieces;
+    for (int p0 = first_pair, left = n_pairs, quarters = 1; left > 0; quarters = std::min(2 * quarters, cap)) {
+        int np = q * quarters;
+        if ((int)pieces.size() >= SEQ_MAX_GROUPS - 1 || left - np < q) np = left;     // else np < left
+        pieces.emplace_back(p0, np);
+        p0 += np;
+        left -= np;
+    }
+    return pieces;
 }
 
 // After recoverPose: the reference's sanity fallbacks, LM input assembly (first lm_points
@@ -429,7 +463,6 @@ int epivo_seq_create_pairs(epivo_ctx* ctx, epivo_seq** out, int max_frames, int 
     s->max_pairs = max_pairs;
     s->n_list = max_frames - 1;
     const size_t F = max_frames, P = max_pairs, st = s->stride, kp = kp_per_frame;
-    s->chunk = (int)std::min<size_t>(SEQ_CHUNK, P);
     const size_t C = P;        // group-scoped buffers are allocated for every pair, so groups never alias
     int rc = 0;
 #define A(ptr, count) if (!rc) rc = seq_alloc(s, &s->ptr, (count))
@@ -453,28 +486,19 @@ int epivo_seq_create_pairs(epivo_ctx* ctx, epivo_seq** out, int max_frames, int 
 #undef A
     if (!rc && cudaMallocHost(&s->h_results, P * sizeof(epivo_pair_result)) != cudaSuccess) rc = EPIVO_ERR_CUDA;
     bool ev_ok = true;
-    for (int c = 0; c < SEQ_MAX_CHUNKS && ev_ok; ++c)
+    SeqEventArray evs[SEQ_EVENT_ARRAYS];
+    seq_event_arrays(s, evs);
+    for (const SeqEventArray& a : evs)
+        for (int i = 0; i < a.n && ev_ok; ++i) ev_ok = cudaEventCreateWithFlags(&a.ev[i], a.flags) == cudaSuccess;
     {
-        for (int k = 0; k < SEQ_STAGES; ++k) ev_ok &= cudaEventCreate(&s->ev[c][k]) == cudaSuccess;
-        for (int k = 0; k < 2; ++k) ev_ok &= cudaEventCreate(&s->evk[c][k]) == cudaSuccess;
-        ev_ok &= cudaEventCreate(&s->evp[c]) == cudaSuccess;
-    }
-    for (int c = 0; c < SEQ_MAX_CHUNKS && ev_ok; ++c)
-        ev_ok &= cudaEventCreateWithFlags(&s->ev_matched[c], cudaEventDisableTiming) == cudaSuccess;
-    ev_ok = ev_ok && cudaEventCreate(&s->ev_begin) == cudaSuccess && cudaEventCreate(&s->ev_end) == cudaSuccess;
-    ev_ok = ev_ok && cudaEventCreateWithFlags(&s->ev_geo_done, cudaEventDisableTiming) == cudaSuccess;
-    {
-        // the second stream carries the H2D pieces of the host-buffer path and, in overlap mode, the geometry
-        // kernels: highest priority, so that their short CTAs take the SM slots the long matcher CTAs free up
+        // The copy stream's only kernel is the HAMMING2 plane conversion behind each upload piece, and the matcher
+        // launch of that piece waits for it: highest priority, so that its CTAs take the first SM slots the draining
+        // matcher CTAs free up instead of queueing behind the next matcher wave.  Its effect on the plane kernel
+        // alone has not been measured.
         int lo = 0, hi = 0;
         cudaDeviceGetStreamPriorityRange(&lo, &hi);       // hi = numerically lowest = highest priority
         ev_ok = ev_ok && cudaStreamCreateWithPriority(&s->stream2, cudaStreamNonBlocking, hi) == cudaSuccess;
         ev_ok = ev_ok && cudaStreamCreateWithFlags(&s->stream3, cudaStreamNonBlocking) == cudaSuccess;
-        // highest priority: a geometry kernel is a chain of ~70 short dependent launches; behind a resident wave of
-        // 0.9 ms matcher CTAs each of them would wait for a free slot at normal priority
-        ev_ok = ev_ok && cudaStreamCreateWithPriority(&s->stream4, cudaStreamNonBlocking, hi) == cudaSuccess;
-        for (int c = 0; c < SEQ_MAX_CHUNKS && ev_ok; ++c)
-            ev_ok &= cudaEventCreateWithFlags(&s->ev_piece[c], cudaEventDisableTiming) == cudaSuccess;
     }
     if (rc || !ev_ok) {
         epivo_seq_destroy(s);
@@ -502,24 +526,13 @@ void epivo_seq_destroy(epivo_seq* s) {
     cudaStreamSynchronize(s->ctx->stream);
     for (void* p : s->allocs) cudaFree(p);
     if (s->h_results) cudaFreeHost(s->h_results);
-    for (int c = 0; c < SEQ_MAX_CHUNKS; ++c)
-        for (int k = 0; k < SEQ_STAGES; ++k)
-            if (s->ev[c][k]) cudaEventDestroy(s->ev[c][k]);
-    for (int c = 0; c < SEQ_MAX_CHUNKS; ++c)
-        for (int k = 0; k < 2; ++k)
-            if (s->evk[c][k]) cudaEventDestroy(s->evk[c][k]);
-    for (int c = 0; c < SEQ_MAX_CHUNKS; ++c)
-        if (s->evp[c]) cudaEventDestroy(s->evp[c]);
-    for (int c = 0; c < SEQ_MAX_CHUNKS; ++c)
-        if (s->ev_matched[c]) cudaEventDestroy(s->ev_matched[c]);
-    if (s->ev_geo_done) cudaEventDestroy(s->ev_geo_done);
     if (s->stream2) { cudaStreamSynchronize(s->stream2); cudaStreamDestroy(s->stream2); }
     if (s->stream3) { cudaStreamSynchronize(s->stream3); cudaStreamDestroy(s->stream3); }
-    if (s->stream4) { cudaStreamSynchronize(s->stream4); cudaStreamDestroy(s->stream4); }
-    for (int c = 0; c < SEQ_MAX_CHUNKS; ++c)
-        if (s->ev_piece[c]) cudaEventDestroy(s->ev_piece[c]);
-    if (s->ev_begin) cudaEventDestroy(s->ev_begin);
-    if (s->ev_end) cudaEventDestroy(s->ev_end);
+    SeqEventArray evs[SEQ_EVENT_ARRAYS];
+    seq_event_arrays(s, evs);
+    for (const SeqEventArray& a : evs)
+        for (int i = 0; i < a.n; ++i)
+            if (a.ev[i]) cudaEventDestroy(a.ev[i]);
     delete s;
 }
 
@@ -642,20 +655,14 @@ int epivo_seq_extract_orb(epivo_seq* s, int first_frame, int n_frames, const uin
     return EPIVO_OK;
 }
 
-int epivo_seq_set_overlap(epivo_seq* s, int overlap) {
-    if (!s) return EPIVO_ERR_INVALID;
-    s->overlap = overlap == 1 ? 1 : 0;
-    s->geo_mode = overlap == 2 ? 2 : 0;
-    return EPIVO_OK;
-}
-
-// geometry of one group on the context's CURRENT stream (the caller selects the stream)
+// geometry of one group on the context stream
 static int seq_run_geometry(epivo_seq* s, const epivo_pipeline_params* prm, int c, int p0, int np) {
     epivo_ctx* ctx = s->ctx;
     const int st = s->stride;
     const size_t o = (size_t)p0;                 // group-scoped buffers are indexed by absolute pair
+    cudaEvent_t* ev = s->ev_geo[c];
     int rc;
-    EPV_CUDA(ctx, cudaEventRecord(s->ev[c][2], ctx->stream));
+    EPV_CUDA(ctx, cudaEventRecord(ev[0], ctx->stream));
     EpvRange r_geo(ctx, "epivo: geometry (findEssentialMat + recoverPose + LM)");
     EssentialPlan ep{};
     ep.n_pairs = np;
@@ -678,13 +685,13 @@ static int seq_run_geometry(epivo_seq* s, const epivo_pipeline_params* prm, int 
     ep.xin = s->d_xin + o * 4 * st;
     ep.work = s->d_esswork;          // one group at a time uses it: groups are stream-ordered
     ep.work_bytes = s->esswork_bytes;
-    ep.ev_presolved = s->evp[c];
+    ep.ev_presolved = ev[5];
     {
         EpvRange r(ctx, "epivo: findEssentialMat");
         rc = epv_essential_launch(ctx, ep);
     }
     if (rc) return rc;
-    EPV_CUDA(ctx, cudaEventRecord(s->ev[c][3], ctx->stream));
+    EPV_CUDA(ctx, cudaEventRecord(ev[1], ctx->stream));
     PosePlan pp{};
     pp.n_pairs = np;
     pp.stride = st;
@@ -703,7 +710,7 @@ static int seq_run_geometry(epivo_seq* s, const epivo_pipeline_params* prm, int 
         rc = epv_pose_launch(ctx, pp);
     }
     if (rc) return rc;
-    EPV_CUDA(ctx, cudaEventRecord(s->ev[c][4], ctx->stream));
+    EPV_CUDA(ctx, cudaEventRecord(ev[2], ctx->stream));
     lm_prep_kernel<<<np, 64, 0, ctx->stream>>>(np, st, *prm, s->d_R + o * 9, s->d_t + o * 3, s->d_status + p0,
                                                s->d_ninl + p0, s->d_ngood + p0, s->d_xin + o * 4 * st,
                                                s->d_T0 + o * 16, s->d_T + o * 16, s->d_lmp + o * 64 * 3,
@@ -732,13 +739,13 @@ static int seq_run_geometry(epivo_seq* s, const epivo_pipeline_params* prm, int 
         rc = epv_lm_launch(ctx, lp);
     }
     if (rc) return rc;
-    EPV_CUDA(ctx, cudaEventRecord(s->ev[c][5], ctx->stream));
+    EPV_CUDA(ctx, cudaEventRecord(ev[3], ctx->stream));
     finish_kernel<<<(np + 127) / 128, 128, 0, ctx->stream>>>(
         np, *prm, s->d_E + o * 9, s->d_R + o * 9, s->d_t + o * 3, s->d_T0 + o * 16, s->d_T + o * 16, s->d_lmres + p0,
         s->d_lmiters + p0, s->d_lmactive + p0, s->d_nmatch + p0, s->d_ninl + p0, s->d_ngood + p0, s->d_iters + p0,
         s->d_nmodels + p0, s->d_results + p0);
     EPV_LAUNCHED(ctx);
-    EPV_CUDA(ctx, cudaEventRecord(s->ev[c][6], ctx->stream));
+    EPV_CUDA(ctx, cudaEventRecord(ev[4], ctx->stream));
     return EPIVO_OK;
 }
 
@@ -747,8 +754,9 @@ static int seq_run_match(epivo_seq* s, const epivo_pipeline_params* prm, int c, 
     epivo_ctx* ctx = s->ctx;
     const int kp = s->kp, st = s->stride;
     const size_t o = (size_t)p0;
+    cudaEvent_t* ev = s->ev_match[c];
     int rc;
-    EPV_CUDA(ctx, cudaEventRecord(s->ev[c][0], ctx->stream));
+    EPV_CUDA(ctx, cudaEventRecord(ev[0], ctx->stream));
     EpvRange r_match(ctx, "epivo: BFMatcher::match");
     MatchPlan mp{};
     mp.desc = s->d_desc + o * kp * 8;                     // group-local view: frames p0 .. p0+np
@@ -771,9 +779,8 @@ static int seq_run_match(epivo_seq* s, const epivo_pipeline_params* prm, int c, 
     mp.rowkey2 = s->d_rowkey2 + o * st;
     mp.colkey = s->d_colkey + o * st;
     mp.stride = st;
-    mp.ev0 = s->evk[c][0];
-    mp.ev1 = s->evk[c][1];
-    mp.pad_smem = s->match_pad;
+    mp.ev0 = ev[2];
+    mp.ev1 = ev[3];
     const bool general = s->counts_set || s->pairs_set;     // per-frame counts and / or an explicit pair list
     bool prepass = true;
     if (general) {
@@ -793,7 +800,7 @@ static int seq_run_match(epivo_seq* s, const epivo_pipeline_params* prm, int c, 
     if (planes_ready) prepass = false;                      // converted on the copy stream, piece by piece
     rc = epv_match_launch(ctx, mp, prepass);
     if (rc) return rc;
-    EPV_CUDA(ctx, cudaEventRecord(s->ev[c][1], ctx->stream));
+    EPV_CUDA(ctx, cudaEventRecord(ev[1], ctx->stream));
     FinalizePlan fp{};
     fp.n_pairs = np;
     fp.nq = kp;
@@ -834,102 +841,85 @@ static int seq_run_match(epivo_seq* s, const epivo_pipeline_params* prm, int c, 
     return EPIVO_OK;
 }
 
-// Tuning aid (EPIVO_UPLOAD_DELAY_US): a sleeping kernel on the copy stream behind every upload piece, to reproduce on
-// one GPU the input rate a rank sees when eight ranks share the host's copy path.
-__device__ __forceinline__ unsigned long long epv_globaltimer_ns() {
-    unsigned long long t;
-    asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(t));
-    return t;
-}
-__global__ void upload_delay_kernel(unsigned us) {
-    const unsigned long long t0 = epv_globaltimer_ns();
-    while (epv_globaltimer_ns() - t0 < (unsigned long long)us * 1000ull) __nanosleep(2000);
+// Checks every run through the geometry makes before its first launch: the geometry parameters, and no more pair
+// groups than event slots.
+static int seq_check_geometry(epivo_seq* s, const epivo_pipeline_params* prm, int n_pairs) {
+    epivo_ctx* ctx = s->ctx;
+    if (prm->lm_points < 1 || prm->lm_points > 64) EPV_FAIL(ctx, EPIVO_ERR_UNSUPPORTED, "lm_points must be in [1,64]");
+    if (prm->method != EPIVO_RANSAC && prm->method != EPIVO_LMEDS) EPV_FAIL(ctx, EPIVO_ERR_INVALID, "method");
+    if ((n_pairs + SEQ_CHUNK - 1) / SEQ_CHUNK > SEQ_MAX_GROUPS) EPV_FAIL(ctx, EPIVO_ERR_UNSUPPORTED, "too many pair groups");
+    return EPIVO_OK;
 }
 
-// Common executor.  With host buffers (h_kps/h_desc != NULL) the frames are uploaded in pieces on
-// the copy stream and every matcher group starts as soon as its frames have landed, so the
-// host->device transfer hides under the matcher; the geometry then runs once over all pairs.
+// The pairs a call over n_frames frames from the host runs: the whole pair list (every frame it references must be
+// given), or the consecutive pairs (p, p + 1).
+static int seq_frame_pairs(epivo_seq* s, int n_frames, int* n_pairs) {
+    if (s->pairs_set && s->list_max >= n_frames)
+        EPV_FAIL(s->ctx, EPIVO_ERR_INVALID, "the pair list references frame %d but only %d frames are given", s->list_max,
+                 n_frames);
+    *n_pairs = s->pairs_set ? s->n_list : n_frames - 1;
+    return EPIVO_OK;
+}
+
+// What the run being enqueued leaves on the device, for epivo_seq_stage_ms / _cloud / _get_points / _bundle_adjust.
+static void seq_set_last_run(epivo_seq* s, epivo_seq::RunKind run, int first_pair, int n_pairs, int mgroups) {
+    s->last_run = run;
+    s->last_frames = run == epivo_seq::RUN_FRAMES;
+    s->last_first = first_pair;
+    s->last_n_pairs = n_pairs;
+    s->last_mgroups = mgroups;
+}
+
+// The geometry of pairs [first_pair, +n_pairs) in groups of SEQ_CHUNK on the context stream, after whatever produced
+// their correspondences there; ev_end closes the run.  It runs after all of the matcher: running it under the matcher
+// or between the upload pieces measured slower in every regime (DESIGN.md section 4 "Pipeline" and section 6).
+static int seq_geometry(epivo_seq* s, const epivo_pipeline_params* prm, int first_pair, int n_pairs) {
+    epivo_ctx* ctx = s->ctx;
+    const int n_g = (n_pairs + SEQ_CHUNK - 1) / SEQ_CHUNK;
+    s->last_ggroups = n_g;
+    for (int c = 0; c < n_g; ++c) {
+        const int p0 = first_pair + c * SEQ_CHUNK;
+        const int rc = seq_run_geometry(s, prm, c, p0, std::min(SEQ_CHUNK, first_pair + n_pairs - p0));
+        if (rc) return rc;
+    }
+    EPV_CUDA(ctx, cudaEventRecord(s->ev_end, ctx->stream));
+    return EPIVO_OK;
+}
+
+// Common executor of epivo_seq_run and epivo_seq_process.  Resident frames: matcher groups of SEQ_CHUNK pairs on the
+// context stream.  Host buffers (h_kps/h_desc != NULL): the frames are uploaded in pieces on the copy stream and every
+// matcher piece starts as soon as its frames have landed, so the host->device transfer hides under the matcher; with
+// a pair list, which may reference any frame, the upload goes whole before the first group.  The geometry then runs
+// once over all pairs.
 static int seq_execute(epivo_seq* s, const epivo_pipeline_params* prm, int first_pair, int n_pairs,
                        const float* h_kps, const uint8_t* h_desc, int n_frames_up) {
     epivo_ctx* ctx = s->ctx;
     if (first_pair < 0 || n_pairs < 0 || first_pair + n_pairs > s->n_list)
         EPV_FAIL(ctx, EPIVO_ERR_INVALID, "pair range [%d,+%d) outside [0,%d)", first_pair, n_pairs, s->n_list);
-    if (prm->lm_points < 1 || prm->lm_points > 64) EPV_FAIL(ctx, EPIVO_ERR_UNSUPPORTED, "lm_points must be in [1,64]");
-    if (prm->method != EPIVO_RANSAC && prm->method != EPIVO_LMEDS) EPV_FAIL(ctx, EPIVO_ERR_INVALID, "method");
+    int rc = seq_check_geometry(s, prm, n_pairs);
+    if (rc) return rc;
     if (prm->match_mode < 0 || prm->match_mode > 2) EPV_FAIL(ctx, EPIVO_ERR_INVALID, "match_mode");
     if (prm->norm != EPIVO_NORM_HAMMING && prm->norm != EPIVO_NORM_HAMMING2) EPV_FAIL(ctx, EPIVO_ERR_INVALID, "norm");
     EPV_CUDA(ctx, cudaSetDevice(ctx->device));
     cudaStream_t main_stream = ctx->stream;
     EpvRange r_seq(ctx, h_kps ? "epivo_seq_process" : "epivo_seq_run");
-    // an explicit pair list may reference any frame: host buffers are then uploaded whole before the first group
     const bool upload_all = h_kps != nullptr && s->pairs_set;
     const bool upload = h_kps != nullptr && !upload_all;
-    const bool overlap = s->overlap && !upload && !upload_all;
-    if (upload || upload_all) s->frames_hi = std::max(s->frames_hi, first_pair + n_frames_up);
+    if (h_kps) s->frames_hi = std::max(s->frames_hi, first_pair + n_frames_up);
     if (s->pairs_set && s->frames_hi == 0) EPV_FAIL(ctx, EPIVO_ERR_INVALID, "pair list set but no frames uploaded");
     if (s->pairs_set && s->list_max >= s->frames_hi)          // a slot never uploaded would be matched as garbage
         EPV_FAIL(ctx, EPIVO_ERR_INVALID, "the pair list references frame %d but only frames [0,%d) have been uploaded",
                  s->list_max, s->frames_hi);
-    // matcher groups / geometry groups (event slots: matcher [0, HALF), geometry [HALF, 2*HALF))
-    constexpr int HALF = SEQ_MAX_CHUNKS / 2;
-    // matcher groups.  Resident data: uniform groups.  Host buffers: the upload is cut into pieces of at most one wave
-    // of matcher CTAs, every matcher launch waiting only for its own frames (and the launches alternate between
-    // two streams, see below, so a piece boundary costs nothing).  Small pieces are what matters when the copy is
-    // slower than the matcher: alone on a box the PCIe copy delivers frames 2x faster than the matcher consumes
-    // them (55 GB/s against 26 GB/s) and any schedule hides it, but with eight ranks pulling at once a rank gets
-    // 23 GB/s (profiles/r2_h2d_ceiling_8gpu.json), the matcher runs behind the copy, and the step ends one piece
-    // of matching after the last byte lands (round 1's 1, 2, 4, rest schedule left 2468 pairs = 7.5 ms there).
-    std::vector<std::pair<int, int> > mg;     // (first pair, pairs)
-    {
-        const int mchunk = overlap ? SEQ_CHUNK_OVERLAP : SEQ_CHUNK;
-        int wave = upload ? epv_match_pairs_per_wave(ctx, s->kp) : mchunk;
-        int max_pieces = HALF, cap_waves = 4;
-        if (upload) {                                   // tuning knobs (environment): first piece = wave / div, piece count, cap
-            // default: a quarter wave first (the matcher starts 0.1 ms after the call instead of 0.43), doubling up to
-            // one wave: 74, 148, 296, 296, ... pairs (measured 17.17 -> 16.94 ms per step against 16.65 device-resident)
-            int div = 4;
-            if (const char* e = getenv("EPIVO_UPLOAD_DIV")) div = std::max(1, atoi(e));
-            wave = std::max(1, wave / div);
-            if (const char* e = getenv("EPIVO_UPLOAD_PIECES")) max_pieces = std::min(HALF, std::max(1, atoi(e)));
-            if (const char* e = getenv("EPIVO_UPLOAD_CAP")) cap_waves = std::max(1, atoi(e));
-            // never more pieces than event slots: widen the cap for very long sequences
-            while ((n_pairs + (int64_t)wave * cap_waves - 1) / ((int64_t)wave * cap_waves) + 2 > max_pieces && cap_waves < (1 << 20))
-                cap_waves *= 2;
-        }
-        int p0 = first_pair, left = n_pairs, waves = 1;
-        while (left > 0) {
-            int np = upload ? wave * waves : mchunk;
-            if (upload && ((int)mg.size() >= max_pieces - 1 || left - np < wave)) np = left;    // the last piece takes the rest
-            np = std::min(np, left);
-            mg.push_back(std::make_pair(p0, np));
-            p0 += np;
-            left -= np;
-            waves = std::min(2 * waves, cap_waves);
-        }
+    std::vector<std::pair<int, int> > mg;     // matcher groups: (first pair, pairs)
+    if (upload) {
+        mg = seq_upload_pieces(first_pair, n_pairs, epv_match_pairs_per_wave(ctx, s->kp));
+    } else {
+        for (int p0 = first_pair; p0 < first_pair + n_pairs; p0 += SEQ_CHUNK)
+            mg.emplace_back(p0, std::min(SEQ_CHUNK, first_pair + n_pairs - p0));
     }
-    const int gchunk = overlap ? SEQ_CHUNK_OVERLAP : SEQ_CHUNK;
-    const int n_m = (int)mg.size(), n_g = (n_pairs + gchunk - 1) / gchunk;
-    if (n_m > HALF || n_g > HALF) EPV_FAIL(ctx, EPIVO_ERR_UNSUPPORTED, "too many pair groups");
-    s->last_mgroups = n_m;
-    s->last_ggroups = n_g;
-    s->last_frames = false;
-    s->last_run = epivo_seq::RUN_DESC;
-    s->last_n_pairs = n_pairs;
-    s->last_first = first_pair;
-    // Host-buffer path: the geometry of the pairs already matched CAN run between the matcher pieces (four groups, own
-    // high-priority stream: epivo_seq_set_overlap(seq, 2)), which looks attractive when the copy is the limiter and
-    // the GPU idles between pieces.  Measured, it loses in every regime -- 17.2 -> 18.9 ms per step with the copy at
-    // full rate, 22.4 -> 23.1 ms with the copy throttled to the rate of an 8-rank run (EPIVO_UPLOAD_DELAY_US), and
-    // 19.7 -> 20.8 ms on 8 GPUs: a geometry group is a chain of ~70 short dependent launches whose CTAs take slots
-    // and issue cycles from the matcher wave that has just become ready, and the matcher then falls behind the copy.
-    // So the default stays: geometry after the last matcher piece.
-    int geo_mode = s->geo_mode;
-    if (const char* e = getenv("EPIVO_GEO_MODE")) geo_mode = atoi(e);      // tuning / experiments: 2 = interleave
-    const bool interleave = upload && n_m >= 8 && geo_mode == 2;
-    if (upload && getenv("EPIVO_DEBUG_SCHED"))
-        fprintf(stderr, "[epivo dev %d] host-buffer call: %d pieces, interleave %d\n", ctx->device, n_m, (int)interleave);
+    const int n_m = (int)mg.size();           // <= SEQ_MAX_GROUPS: seq_check_geometry / seq_upload_pieces
+    seq_set_last_run(s, epivo_seq::RUN_DESC, first_pair, n_pairs, n_m);
     EPV_CUDA(ctx, cudaEventRecord(s->ev_begin, main_stream));
-    int rc = EPIVO_OK;
     const size_t kp = s->kp;
     const bool planes_on_copy = upload && prm->norm == EPIVO_NORM_HAMMING2;
     if (upload) {
@@ -938,8 +928,6 @@ static int seq_execute(epivo_seq* s, const epivo_pipeline_params* prm, int first
         // depends on nothing but its own event (no pre-pass in front of it, no frame converted twice).
         EPV_CUDA(ctx, cudaStreamWaitEvent(s->stream2, s->ev_begin, 0));
         EPV_CUDA(ctx, cudaStreamWaitEvent(s->stream3, s->ev_begin, 0));
-        const char* de = getenv("EPIVO_UPLOAD_DELAY_US");
-        const int delay_us = de ? atoi(de) : 0;
         for (int c = 0; c < n_m; ++c) {
             const int p0 = mg[c].first, np = mg[c].second;
             const int f0 = (c == 0) ? p0 : p0 + 1;                  // frame p0 came with the previous piece
@@ -954,80 +942,35 @@ static int seq_execute(epivo_seq* s, const epivo_pipeline_params* prm, int first
                                        (int64_t)nf * kp, 8, s->stream2);
                 if (rc) return rc;
             }
-            if (delay_us > 0) upload_delay_kernel<<<1, 1, 0, s->stream2>>>((unsigned)delay_us);
-            EPV_CUDA(ctx, cudaEventRecord(s->ev_matched[c], s->stream2));
+            EPV_CUDA(ctx, cudaEventRecord(s->ev_landed[c], s->stream2));
         }
-        if (interleave) EPV_CUDA(ctx, cudaStreamWaitEvent(s->stream4, s->ev_begin, 0));
     }
     if (upload_all) {
         EPV_CUDA(ctx, cudaStreamWaitEvent(s->stream2, s->ev_begin, 0));
         EPV_CUDA(ctx, cudaMemcpyAsync(s->d_kps, h_kps, (size_t)n_frames_up * kp * 8, cudaMemcpyHostToDevice, s->stream2));
         EPV_CUDA(ctx, cudaMemcpyAsync(s->d_desc, h_desc, (size_t)n_frames_up * kp * 32, cudaMemcpyHostToDevice, s->stream2));
-        EPV_CUDA(ctx, cudaEventRecord(s->ev_matched[0], s->stream2));
-        EPV_CUDA(ctx, cudaStreamWaitEvent(main_stream, s->ev_matched[0], 0));
+        EPV_CUDA(ctx, cudaEventRecord(s->ev_landed[0], s->stream2));
+        EPV_CUDA(ctx, cudaStreamWaitEvent(main_stream, s->ev_landed[0], 0));
     }
-    if (overlap) EPV_CUDA(ctx, cudaStreamWaitEvent(s->stream2, s->ev_begin, 0));
-    int n_geo = 0;                       // geometry groups already issued (interleaved mode)
-    for (int c = 0; c < n_m && !rc; ++c) {
-        const int p0 = mg[c].first, np = mg[c].second;
+    for (int c = 0; c < n_m; ++c) {
         cudaStream_t piece_stream = main_stream;
         if (upload) {
             // the matcher pieces alternate between two streams: piece c+1 (its frames have landed) fills the SMs
             // that the draining CTAs of piece c free up, and its finalize / key-fill kernels run beside piece c+1's
             // tiles -- on one stream every piece boundary cost ~0.1 ms of drained GPU
             piece_stream = (c & 1) ? s->stream3 : main_stream;
-            EPV_CUDA(ctx, cudaStreamWaitEvent(piece_stream, s->ev_matched[c], 0));
+            EPV_CUDA(ctx, cudaStreamWaitEvent(piece_stream, s->ev_landed[c], 0));
         }
         ctx->stream = piece_stream;
-        rc = seq_run_match(s, prm, c, p0, np, planes_on_copy);
+        rc = seq_run_match(s, prm, c, mg[c].first, mg[c].second, planes_on_copy);
         ctx->stream = main_stream;
-        if (rc) break;
-        if (interleave) {
-            EPV_CUDA(ctx, cudaEventRecord(s->ev_piece[c], piece_stream));
-            const int per = (n_m + 3) / 4;                          // pieces per geometry group
-            if ((c + 1) % per == 0 || c == n_m - 1) {
-                const int c0 = (c / per) * per;                     // the group's first piece
-                const int gp0 = mg[c0].first, gnp = p0 + np - gp0;
-                EPV_CUDA(ctx, cudaStreamWaitEvent(s->stream4, s->ev_piece[c], 0));
-                if (c > 0) EPV_CUDA(ctx, cudaStreamWaitEvent(s->stream4, s->ev_piece[c - 1], 0));   // the other stream's last piece
-                ctx->stream = s->stream4;
-                rc = seq_run_geometry(s, prm, HALF + n_geo, gp0, gnp);
-                ctx->stream = main_stream;
-                if (rc) break;
-                ++n_geo;
-            }
-        }
-        if (overlap) {      // optional two-stream compute: geometry of group c under the matcher of c+1
-            EPV_CUDA(ctx, cudaEventRecord(s->ev_matched[c], main_stream));
-            EPV_CUDA(ctx, cudaStreamWaitEvent(s->stream2, s->ev_matched[c], 0));
-            ctx->stream = s->stream2;
-            rc = seq_run_geometry(s, prm, HALF + c, p0, np);
-            ctx->stream = main_stream;
-        }
-    }
-    if (upload && n_m > 1 && !rc) {     // the odd pieces join the context stream before the geometry
-        EPV_CUDA(ctx, cudaEventRecord(s->ev_geo_done, s->stream3));
-        EPV_CUDA(ctx, cudaStreamWaitEvent(main_stream, s->ev_geo_done, 0));
-    }
-    ctx->stream = main_stream;
-    if (rc) return rc;
-    if (interleave) {       // every group's geometry is already queued on stream4: join it
-        s->last_ggroups = n_geo;
-        EPV_CUDA(ctx, cudaEventRecord(s->ev_geo_done, s->stream4));
-        EPV_CUDA(ctx, cudaStreamWaitEvent(main_stream, s->ev_geo_done, 0));
-    } else if (overlap) {   // later work on the context stream (download) is ordered after the geometry
-        EPV_CUDA(ctx, cudaEventRecord(s->ev_geo_done, s->stream2));
-        EPV_CUDA(ctx, cudaStreamWaitEvent(main_stream, s->ev_geo_done, 0));
-    } else {
-        for (int c = 0; c < n_g && !rc; ++c) {
-            const int p0 = first_pair + c * gchunk;
-            const int np = std::min(gchunk, first_pair + n_pairs - p0);
-            rc = seq_run_geometry(s, prm, HALF + c, p0, np);
-        }
         if (rc) return rc;
     }
-    EPV_CUDA(ctx, cudaEventRecord(s->ev_end, main_stream));
-    return EPIVO_OK;
+    if (upload && n_m > 1) {     // the odd pieces join the context stream before the geometry
+        EPV_CUDA(ctx, cudaEventRecord(s->ev_join, s->stream3));
+        EPV_CUDA(ctx, cudaStreamWaitEvent(main_stream, s->ev_join, 0));
+    }
+    return seq_geometry(s, prm, first_pair, n_pairs);
 }
 
 int epivo_seq_run(epivo_seq* s, const epivo_pipeline_params* prm, int first_pair, int n_pairs) {
@@ -1041,11 +984,10 @@ int epivo_seq_process(epivo_seq* s, const epivo_pipeline_params* prm, int n_fram
     epivo_ctx* ctx = s->ctx;
     if (!kps || !descs || !out) EPV_FAIL(ctx, EPIVO_ERR_INVALID, "null buffer");
     if (n_frames < 2 || n_frames > s->max_frames) EPV_FAIL(ctx, EPIVO_ERR_INVALID, "n_frames %d outside [2,%d]", n_frames, s->max_frames);
-    // consecutive pairs: n_frames - 1 of them; explicit pair list (epivo_seq_set_pairs): the whole list
-    if (s->pairs_set && s->list_max >= n_frames)
-        EPV_FAIL(ctx, EPIVO_ERR_INVALID, "the pair list references frame %d but only %d frames are given", s->list_max, n_frames);
-    const int n_pairs = s->pairs_set ? s->n_list : n_frames - 1;
-    int rc = seq_execute(s, prm, 0, n_pairs, kps, descs, n_frames);
+    int n_pairs = 0;
+    int rc = seq_frame_pairs(s, n_frames, &n_pairs);
+    if (rc) return rc;
+    rc = seq_execute(s, prm, 0, n_pairs, kps, descs, n_frames);
     if (rc) return rc;
     return epivo_seq_download(s, out, 0, n_pairs);
 }
@@ -1058,14 +1000,14 @@ int epivo_seq_process_points(epivo_seq* s, const epivo_pipeline_params* prm, int
     if (n_pairs == 0) return EPIVO_OK;
     if (!p0 || !p1 || !counts || !out) EPV_FAIL(ctx, EPIVO_ERR_INVALID, "null buffer");
     if (max_pts < 1 || max_pts > s->kp) EPV_FAIL(ctx, EPIVO_ERR_INVALID, "max_pts %d outside [1,%d]", max_pts, s->kp);
-    if (prm->lm_points < 1 || prm->lm_points > 64) EPV_FAIL(ctx, EPIVO_ERR_UNSUPPORTED, "lm_points must be in [1,64]");
-    if (prm->method != EPIVO_RANSAC && prm->method != EPIVO_LMEDS) EPV_FAIL(ctx, EPIVO_ERR_INVALID, "method");
+    int rc = seq_check_geometry(s, prm, n_pairs);
+    if (rc) return rc;
     for (int i = 0; i < n_pairs; ++i)
         if (counts[i] < 0 || counts[i] > max_pts) EPV_FAIL(ctx, EPIVO_ERR_INVALID, "counts[%d] = %d outside [0,%d]", i, counts[i], max_pts);
     EPV_CUDA(ctx, cudaSetDevice(ctx->device));
     EpvRange r_seq(ctx, "epivo_seq_process_points");
     const size_t np = (size_t)n_pairs * max_pts;
-    int rc = epv_ws_reserve(ctx, np * 16 + (size_t)n_pairs * 4 + 4096);
+    rc = epv_ws_reserve(ctx, np * 16 + (size_t)n_pairs * 4 + 4096);
     if (rc) return rc;
     float* d_p0 = epv_ws_take<float>(ctx, np * 2);
     float* d_p1 = epv_ws_take<float>(ctx, np * 2);
@@ -1080,21 +1022,9 @@ int epivo_seq_process_points(epivo_seq* s, const epivo_pipeline_params* prm, int
                                                                             -prm->K[2] * ax, ay, -prm->K[5] * ay, s->d_xn,
                                                                             s->d_nmatch, s->d_mq, s->d_mt);
     EPV_LAUNCHED(ctx);
-    constexpr int HALF = SEQ_MAX_CHUNKS / 2;
-    const int n_g = (n_pairs + SEQ_CHUNK - 1) / SEQ_CHUNK;
-    if (n_g > HALF) EPV_FAIL(ctx, EPIVO_ERR_UNSUPPORTED, "too many pair groups");
-    s->last_mgroups = 0;
-    s->last_ggroups = n_g;
-    s->last_n_pairs = n_pairs;
-    s->last_first = 0;
-    s->last_frames = false;
-    s->last_run = epivo_seq::RUN_POINTS;
-    for (int c = 0; c < n_g; ++c) {
-        const int g0 = c * SEQ_CHUNK, gn = std::min(SEQ_CHUNK, n_pairs - g0);
-        rc = seq_run_geometry(s, prm, HALF + c, g0, gn);
-        if (rc) return rc;
-    }
-    EPV_CUDA(ctx, cudaEventRecord(s->ev_end, st));
+    seq_set_last_run(s, epivo_seq::RUN_POINTS, 0, n_pairs, 0);
+    rc = seq_geometry(s, prm, 0, n_pairs);
+    if (rc) return rc;
     return epivo_seq_download(s, out, 0, n_pairs);
 }
 
@@ -1104,7 +1034,7 @@ int epivo_seq_process_points(epivo_seq* s, const epivo_pipeline_params* prm, int
 // the pairs of the window and the status compaction into the sequence's correspondence buffers.  Consecutive windows
 // share S = max |ft - fq| frames, so every pair lies inside a window; a pair is tracked in the first window that holds
 // both of its frames.  The geometry then runs over all pairs as in epivo_seq_process_points (not interleaved with the
-// front end: overlapping the geometry with other work measured slower, see epivo_seq_set_overlap).
+// front end: overlapping the geometry with other work measured slower, DESIGN.md section 4 "Pipeline").
 namespace {
 constexpr int FRAMES_MAX_WINDOW = 256;
 constexpr size_t FRAMES_WS_BUDGET = (size_t)3 << 29;        // 1.5 GiB of front-end workspace per window
@@ -1143,14 +1073,11 @@ int epivo_seq_process_frames(epivo_seq* s, const epivo_pipeline_params* prm, int
     if (R <= LK_WINDOW || C <= LK_WINDOW)
         EPV_FAIL(ctx, EPIVO_ERR_UNSUPPORTED, "image %d x %d not larger than the %d x %d LK window", C, R, LK_WINDOW, LK_WINDOW);
     if (fast_threshold < 0 || fast_threshold > 255) EPV_FAIL(ctx, EPIVO_ERR_INVALID, "fast_threshold %d outside [0, 255]", fast_threshold);
-    if (prm->lm_points < 1 || prm->lm_points > 64) EPV_FAIL(ctx, EPIVO_ERR_UNSUPPORTED, "lm_points must be in [1,64]");
-    if (prm->method != EPIVO_RANSAC && prm->method != EPIVO_LMEDS) EPV_FAIL(ctx, EPIVO_ERR_INVALID, "method");
-    if (s->pairs_set && s->list_max >= n_frames)
-        EPV_FAIL(ctx, EPIVO_ERR_INVALID, "the pair list references frame %d but only %d frames are given", s->list_max, n_frames);
-    const int n_pairs = s->pairs_set ? s->n_list : n_frames - 1;
-    constexpr int HALF = SEQ_MAX_CHUNKS / 2;
-    const int n_g = (n_pairs + SEQ_CHUNK - 1) / SEQ_CHUNK;
-    if (n_g > HALF) EPV_FAIL(ctx, EPIVO_ERR_UNSUPPORTED, "too many pair groups");
+    int n_pairs = 0;
+    int rc = seq_frame_pairs(s, n_frames, &n_pairs);
+    if (rc) return rc;
+    rc = seq_check_geometry(s, prm, n_pairs);
+    if (rc) return rc;
     const int kp = s->kp, st = s->stride;
     // window size G: at most 256 frames, and no more than the workspace budget holds
     int G = std::min(FRAMES_MAX_WINDOW, n_frames);
@@ -1187,12 +1114,12 @@ int epivo_seq_process_frames(epivo_seq* s, const epivo_pipeline_params* prm, int
     }
     EPV_CUDA(ctx, cudaSetDevice(ctx->device));
     if (!s->d_trk) {
-        const int rc = seq_alloc(s, &s->d_trk, (size_t)s->max_pairs * st * 4);
+        rc = seq_alloc(s, &s->d_trk, (size_t)s->max_pairs * st * 4);
         if (rc) return rc;
     }
     const FramesWs w = frames_ws(G, rows, cols, R, C, maps, kp);
     const size_t np = (size_t)max_wp * kp;
-    int rc = epv_ws_reserve(ctx, w.total() + epv_align((size_t)n_frames * 4) + epv_align(meta.size() * 4 + 4) +
+    rc = epv_ws_reserve(ctx, w.total() + epv_align((size_t)n_frames * 4) + epv_align(meta.size() * 4 + 4) +
                                      epv_align(np * 8) + epv_align(np) + epv_align(np * 4) + 4096);
     if (rc) return rc;
     uint8_t* d_src = maps ? epv_ws_take<uint8_t>(ctx, w.src) : nullptr;
@@ -1239,18 +1166,9 @@ int epivo_seq_process_frames(epivo_seq* s, const epivo_pipeline_params* prm, int
                                                  s->d_trk, s->d_xn, s->d_nmatch, s->d_mq, s->d_mt, s->d_md);
         EPV_LAUNCHED(ctx);
     }
-    s->last_mgroups = 0;
-    s->last_ggroups = n_g;
-    s->last_n_pairs = n_pairs;
-    s->last_first = 0;
-    s->last_frames = true;
-    s->last_run = epivo_seq::RUN_FRAMES;
-    for (int c = 0; c < n_g; ++c) {
-        const int g0 = c * SEQ_CHUNK, gn = std::min(SEQ_CHUNK, n_pairs - g0);
-        rc = seq_run_geometry(s, prm, HALF + c, g0, gn);
-        if (rc) return rc;
-    }
-    EPV_CUDA(ctx, cudaEventRecord(s->ev_end, cs));
+    seq_set_last_run(s, epivo_seq::RUN_FRAMES, 0, n_pairs, 0);
+    rc = seq_geometry(s, prm, 0, n_pairs);
+    if (rc) return rc;
     if (corners_out) EPV_CUDA(ctx, cudaMemcpyAsync(corners_out, d_found, (size_t)n_frames * 4, cudaMemcpyDeviceToHost, cs));
     return epivo_seq_download(s, out, 0, n_pairs);
 }
@@ -1347,24 +1265,22 @@ int epivo_seq_stage_ms(epivo_seq* s, float* ms, int n) {
     epivo_ctx* ctx = s->ctx;
     EPV_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
     float acc[8] = {0, 0, 0, 0, 0, 0, 0, 0};
-    constexpr int HALF = SEQ_MAX_CHUNKS / 2;
     for (int c = 0; c < s->last_mgroups; ++c) {
+        const cudaEvent_t* ev = s->ev_match[c];
         float t = 0;
-        EPV_CUDA(ctx, cudaEventElapsedTime(&t, s->ev[c][0], s->ev[c][1]));
+        EPV_CUDA(ctx, cudaEventElapsedTime(&t, ev[0], ev[1]));
         acc[1] += t;                // [1] match: plane pre-pass + key init + tile kernel
-        EPV_CUDA(ctx, cudaEventElapsedTime(&t, s->evk[c][0], s->evk[c][1]));
+        EPV_CUDA(ctx, cudaEventElapsedTime(&t, ev[2], ev[3]));
         acc[7] += t;                // [7] matcher tile kernel alone, summed over the group launches
     }
     for (int c = 0; c < s->last_ggroups; ++c) {
-        {                               // [2] sample + presolve (part of [3])
-            float t = 0;
-            EPV_CUDA(ctx, cudaEventElapsedTime(&t, s->ev[HALF + c][2], s->evp[HALF + c]));
-            acc[2] += t;
-        }
-        for (int k = 2; k < 6; ++k) {   // [3] essential [4] pose [5] lm [6] finish
-            float t = 0;
-            EPV_CUDA(ctx, cudaEventElapsedTime(&t, s->ev[HALF + c][k], s->ev[HALF + c][k + 1]));
-            acc[k + 1] += t;
+        const cudaEvent_t* ev = s->ev_geo[c];
+        float t = 0;
+        EPV_CUDA(ctx, cudaEventElapsedTime(&t, ev[0], ev[5]));
+        acc[2] += t;                    // [2] sample + presolve (part of [3])
+        for (int k = 0; k < 4; ++k) {   // [3] essential [4] pose [5] lm [6] finish
+            EPV_CUDA(ctx, cudaEventElapsedTime(&t, ev[k], ev[k + 1]));
+            acc[k + 3] += t;
         }
     }
     float tot = 0;

@@ -278,18 +278,10 @@ int epivo_seq_process_frames(epivo_seq* seq, const epivo_pipeline_params* p, int
 int epivo_seq_get_points(epivo_seq* seq, int pair, float* p0, float* p1, int* n_out);
 /* device -> host copy of the results of the last run and stream sync */
 int epivo_seq_download(epivo_seq* seq, epivo_pair_result* out, int first_pair, int n_pairs);
-/* Scheduling of the geometry (findEssentialMat + recoverPose + LM) relative to the matcher; results do not depend on it.
- *   0 (default)  geometry after the matcher, on the context stream.
- *   1            resident data (epivo_seq_run): groups of pairs pipelined over two streams, the integer-bound matcher of
- *                group g+1 under the FP64-bound geometry of group g.
- *   2            host buffers (epivo_seq_process): the geometry of the pairs already matched runs between the matcher
- *                pieces, in four groups on its own stream.
- * Both alternatives were measured slower than the default on B200 in every regime tried (the geometry kernels take
- * issue slots and registers from the matcher, which holds every SM); they are kept as options, not chosen. */
-int epivo_seq_set_overlap(epivo_seq* seq, int overlap);
 /* per-stage device time of the last run (CUDA events on the context stream), ms:
  * [0] total [1] match [2] presolve (part of 3) [3] essential [4] pose [5] lm [6] finish [7] matcher tile kernel alone
- * [8] number of pair groups; stage times overlap when the two streams do. */
+ * [8] number of pair groups; the geometry runs after the matcher, but epivo_seq_process's matcher pieces alternate
+ * between two streams, so there [1] and [7] count the time two pieces overlap twice. */
 int epivo_seq_stage_ms(epivo_seq* seq, float* ms, int n);
 /* debug/parity views of the last run, host copies: matches of one pair */
 int epivo_seq_get_matches(epivo_seq* seq, int pair, int32_t* query_idx, int32_t* train_idx,

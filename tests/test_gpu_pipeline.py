@@ -70,19 +70,24 @@ def test_sequence_chunking_and_subranges(ctx, seq):
     pipe.close()
 
 
-def test_overlap_on_off_identical(ctx):
-    """Two-stream group pipelining must not change any result (more than one group: 2100 pairs)."""
-    s = synth.make_sequence(n_frames=2101, n=256, seed=synth.seed_for(3, 2))
+def test_run_split_into_groups_identical(ctx):
+    """More pairs than one group of 8192 holds: the run takes two matcher and two geometry groups, and its bytes are
+    those of the same pairs run as two sub-ranges of one group each."""
+    s = synth.make_sequence(n_frames=8201, n=256, seed=synth.seed_for(3, 2))
+    P = s.n_pairs
+    assert P >= 8193
     pipe = api.SequencePipeline(s.n_frames, 256, ctx=ctx)
     pipe.upload(s.kps, s.descs)
     prm = api.default_params(s.K.astype(np.float32))
-    pipe.set_overlap(True)
-    pipe.run(prm, 0, s.n_pairs)
-    a = pipe.download(0, s.n_pairs).copy()
-    pipe.set_overlap(False)
-    pipe.run(prm, 0, s.n_pairs)
-    b = pipe.download(0, s.n_pairs).copy()
-    assert a.tobytes() == b.tobytes()
+    pipe.run(prm, 0, P)
+    a = pipe.download(0, P).copy()
+    assert pipe.stage_ms()[8] == 2
+    h = P // 2
+    pipe.run(prm, 0, h)
+    b0 = pipe.download(0, h).copy()
+    pipe.run(prm, h, P - h)
+    b1 = pipe.download(h, P - h).copy()
+    assert a.tobytes() == b0.tobytes() + b1.tobytes()
     assert (a["n_matches"] > 50).all()
     pipe.close()
 
@@ -101,30 +106,24 @@ def test_process_host_buffers_equals_upload_run_download(ctx):
     pipe2.close()
 
 
-def test_process_geometry_interleaved_or_not_identical(ctx, monkeypatch):
-    """Host-buffer path: many small upload pieces, the geometry between the matcher pieces (mode 2) or after them
-    (default) over repeated calls -- every run must give the bytes of upload + run + download."""
-    monkeypatch.setenv("EPIVO_UPLOAD_DIV", "8")          # 74-pair pieces: 17 of them for 1200 pairs
-    monkeypatch.setenv("EPIVO_UPLOAD_CAP", "1")
-    s = synth.make_sequence(n_frames=1201, n=256, seed=synth.seed_for(3, 5))
-    prm = api.default_params(s.K.astype(np.float32))
+def test_process_many_pieces_identical(ctx):
+    """Host-buffer path with the default upload plan cut into many pieces (at least 8, checked), over repeated calls on
+    one object, and for LMedS and the ratio matcher with plain Hamming (no planes on the copy stream): every call gives
+    the bytes of upload + run + download."""
+    s = synth.make_sequence(n_frames=5001, n=256, seed=synth.seed_for(3, 5))
     ref_pipe = api.SequencePipeline(s.n_frames, 256, ctx=ctx)
     ref_pipe.upload(s.kps, s.descs)
-    ref_pipe.run(prm, 0, s.n_pairs)
-    ref = ref_pipe.download(0, s.n_pairs).tobytes()
-    ref_pipe.close()
     pipe = api.SequencePipeline(s.n_frames, 256, ctx=ctx)
-    for mode in (2, 0, 0, 2):
-        pipe.set_overlap(mode)
-        assert pipe.process(prm, s.kps, s.descs).tobytes() == ref, mode
-    assert pipe.stage_ms()[0] > 0
-    # LMedS, ratio matcher and plain Hamming (no plane pre-pass on the copy stream) through the interleaved form
-    for kw in (dict(method=api.LMEDS, threshold=0.01), dict(norm=api.NORM_HAMMING, match_mode=api.MATCH_RATIO)):
-        p2 = api.default_params(s.K.astype(np.float32), **kw)
-        pipe.set_overlap(0)
-        a = pipe.process(p2, s.kps, s.descs).tobytes()
-        pipe.set_overlap(2)
-        assert pipe.process(p2, s.kps, s.descs).tobytes() == a, kw
+    for i, kw in enumerate((dict(), dict(method=api.LMEDS, threshold=0.01),
+                            dict(norm=api.NORM_HAMMING, match_mode=api.MATCH_RATIO))):
+        prm = api.default_params(s.K.astype(np.float32), **kw)
+        ref_pipe.run(prm, 0, s.n_pairs)
+        ref = ref_pipe.download(0, s.n_pairs).tobytes()
+        for _ in range(3 if i == 0 else 1):
+            assert pipe.process(prm, s.kps, s.descs).tobytes() == ref, kw
+            ms = pipe.stage_ms()
+            assert ms[0] > 0 and ms[8] >= 8, (kw, ms[8])
+    ref_pipe.close()
     pipe.close()
 
 

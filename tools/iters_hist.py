@@ -11,8 +11,6 @@ pipe = api.SequencePipeline(seq.n_frames, 2000, ctx=ctx)
 pipe.upload(seq.kps, seq.descs)
 prm = api.default_params(seq.K.astype(np.float32), threshold=float(os.environ.get("THR", "1.0")),
                          method=api.LMEDS if os.environ.get("LMEDS") else api.RANSAC)
-if os.environ.get("EPIVO_OVERLAP"):
-    pipe.set_overlap(True)
 for _ in range(3):
     pipe.run(prm, 0, seq.n_pairs)
 acc = np.zeros(16)
