@@ -10,9 +10,7 @@ import ctypes as C
 import os
 
 HERE = os.path.dirname(os.path.abspath(__file__))
-# EPIVO_VARIANT selects a tuning build made by build.py with the same variable (default: the product library)
-_VARIANT = os.environ.get("EPIVO_VARIANT", "")
-LIB_PATH = os.path.join(HERE, "libepivo_b200" + ("_" + _VARIANT if _VARIANT else "") + ".so")
+LIB_PATH = os.path.join(HERE, "libepivo_b200.so")
 
 OK, ERR_INVALID, ERR_CUDA, ERR_UNSUPPORTED, ERR_NOMODEL = 0, -1, -2, -3, -4
 NORM_HAMMING, NORM_HAMMING2 = 6, 7

@@ -9,13 +9,11 @@ import sys
 
 HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
-# tuning builds (tools/variants.py): extra -D flags and a different output name / object directory
-_VARIANT = os.environ.get("EPIVO_VARIANT", "")
-OBJ = os.path.join(HERE, "csrc", "build" + ("_" + _VARIANT if _VARIANT else ""))
-LIB = os.path.join(HERE, "libepivo_b200" + ("_" + _VARIANT if _VARIANT else "") + ".so")
+OBJ = os.path.join(HERE, "csrc", "build")
+LIB = os.path.join(HERE, "libepivo_b200.so")
 NVCC = os.environ.get("NVCC", "/usr/local/cuda/bin/nvcc")
 FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-O3", "-std=c++17",
-         "-Xcompiler", "-fPIC", "-Xptxas", "-v"] + os.environ.get("EPIVO_EXTRA_FLAGS", "").split()
+         "-Xcompiler", "-fPIC", "-Xptxas", "-v"]
 # FMA contraction is on: every place that must reproduce OpenCV's un-fused arithmetic bit for bit
 # (Sampson error, K-normalisation) spells its operations with __dmul_rn / __dadd_rn / __fma_rn.
 

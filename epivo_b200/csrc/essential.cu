@@ -12,7 +12,6 @@
 // sequential loop returns.
 #include <float.h>
 #include <math.h>
-#include <stdio.h>
 #include <string.h>
 
 #include <algorithm>
@@ -450,9 +449,7 @@ __global__ void __launch_bounds__(32) solve_a_kernel(EssArgs a, int round, int R
 
 // ---- stage B1: one lane per hypothesis (polynomial + roots); real roots -> compact work list ----
 constexpr int SB1_THREADS = 128;
-#ifndef EPV_SB1_MINBLOCKS
-#define EPV_SB1_MINBLOCKS 4
-#endif
+constexpr int SB1_MINBLOCKS = 4;
 
 // the warp's real roots are appended to the round's item list with one atomic per warp
 __device__ __forceinline__ void append_roots(int count, const double (&zs)[10], uint32_t slot, uint32_t* items,
@@ -490,7 +487,7 @@ __device__ __forceinline__ int reserve_slow(bool want, int32_t* total, int cap) 
     return (want && pos < cap) ? pos : -1;
 }
 
-__global__ void __launch_bounds__(SB1_THREADS, EPV_SB1_MINBLOCKS) solve_b1_kernel(EssArgs a, int round, int R) {
+__global__ void __launch_bounds__(SB1_THREADS, SB1_MINBLOCKS) solve_b1_kernel(EssArgs a, int round, int R) {
     const int count = a.w.ctl[round];
     const int32_t* wl = a.w.wl[round & 1];
     const long long total = (long long)count * R;
@@ -543,11 +540,9 @@ __global__ void __launch_bounds__(SB1_THREADS) solve_b1_slow_kernel(EssArgs a, i
 
 // ---- stage B2: one lane per real root: model + refinement -----------------------------------------
 constexpr int SB2_THREADS = 64;
-#ifndef EPV_SB2_MINBLOCKS
-#define EPV_SB2_MINBLOCKS 4
-#endif
+constexpr int SB2_MINBLOCKS = 4;
 
-__global__ void __launch_bounds__(SB2_THREADS, EPV_SB2_MINBLOCKS) solve_b2_kernel(EssArgs a, int round) {
+__global__ void __launch_bounds__(SB2_THREADS, SB2_MINBLOCKS) solve_b2_kernel(EssArgs a, int round) {
     __shared__ double s_sh[36 * SB2_THREADS];
     const int n_items = a.w.nitems[round];
     for (int it = blockIdx.x * SB2_THREADS + threadIdx.x; it < n_items; it += gridDim.x * SB2_THREADS) {
@@ -569,10 +564,7 @@ __global__ void __launch_bounds__(SB2_THREADS, EPV_SB2_MINBLOCKS) solve_b2_kerne
 // points are staged there, so the loads compile to LDS rather than generic loads)
 // The hot loop is branch-free (pre-filter only); points it cannot decide -- practically none -- are
 // recounted with the exact test in a second loop that is normally skipped.
-#ifndef EPV_ES_UNROLL
-#define EPV_ES_UNROLL 3
-#endif
-constexpr int ES_UNROLL = EPV_ES_UNROLL;   // correspondences in flight per lane in the scoring loops
+constexpr int ES_UNROLL = 3;   // correspondences in flight per lane in the scoring loops
 
 // Inlier counts of two models over the correspondences first, first + step, ... (both models in registers, every
 // correspondence tested against both).
@@ -1074,7 +1066,7 @@ __global__ void __launch_bounds__(32) five_point_a_kernel(const double* __restri
 }
 
 // stage B1 + B2 for the stand-alone solver: flags[i] = valid-model mask, models at fixed positions
-__global__ void __launch_bounds__(SB1_THREADS, EPV_SB1_MINBLOCKS)
+__global__ void __launch_bounds__(SB1_THREADS, SB1_MINBLOCKS)
 five_point_b1_kernel(const double* __restrict__ rec, int m, uint32_t* __restrict__ flags, uint32_t* __restrict__ items,
                      double* __restrict__ item_z, int32_t* __restrict__ n_items) {
     for (long long base = (long long)blockIdx.x * SB1_THREADS; base < m; base += (long long)gridDim.x * SB1_THREADS) {
@@ -1082,26 +1074,14 @@ five_point_b1_kernel(const double* __restrict__ rec, int m, uint32_t* __restrict
         double zs[10];
         int nz = 0;
         if (i < m) {
-#ifdef EPV_ESS_DEBUG
-            double dbg[31];
-            nz = fivept::stage_b1<false>(rec + i, (size_t)m, zs, nullptr, 1, dbg);
-            if (m == 1) {
-                printf("poly asc:");
-                for (int k = 0; k < 11; ++k) printf(" %.17g", dbg[k]);
-                printf("\nroots:");
-                for (int k = 0; k < 10; ++k) printf(" (%.12g, %.3e)", dbg[11 + k], dbg[21 + k]);
-                printf("\nreal roots kept: %d\n", nz);
-            }
-#else
             nz = fivept::stage_b1<false>(rec + i, (size_t)m, zs);                // no state buffer: all sweeps in place
-#endif
             flags[i] = 0;
         }
         append_roots(nz, zs, (uint32_t)i, items, item_z, n_items);
     }
 }
 
-__global__ void __launch_bounds__(SB2_THREADS, EPV_SB2_MINBLOCKS)
+__global__ void __launch_bounds__(SB2_THREADS, SB2_MINBLOCKS)
 five_point_b2_kernel(const double* __restrict__ rec, int m, const uint32_t* __restrict__ items,
                      const double* __restrict__ item_z, const int32_t* __restrict__ n_items, double* __restrict__ Eout,
                      uint32_t* __restrict__ flags) {
@@ -1128,16 +1108,11 @@ constexpr int SC_THREADS = 256;
 // correspondences per thread, in registers: 4, 5 or 6 (template parameter), whichever wastes the fewest point
 // slots for the given n (more independent FP64 chains per thread hide more of the DFMA latency: 6 is preferred)
 constexpr int SC_MODELS = 128;               // models per CTA tile, at most
-#ifndef EPV_SC_KUNROLL
-#define EPV_SC_KUNROLL 1
-#endif
-constexpr int SC_KUNROLL = EPV_SC_KUNROLL;   // models in flight per loop iteration
+constexpr int SC_KUNROLL = 1;   // models in flight per loop iteration
+constexpr int SC_MINBLOCKS = 2;
 
-#ifndef EPV_SC_MINBLOCKS
-#define EPV_SC_MINBLOCKS 2
-#endif
 template <int SC_PPT>
-__global__ void __launch_bounds__(SC_THREADS, EPV_SC_MINBLOCKS)
+__global__ void __launch_bounds__(SC_THREADS, SC_MINBLOCKS)
 score_count_kernel(const double* __restrict__ E, int m, int mtile, const double* __restrict__ xn, int stride, int n,
                    float thr32, int32_t* __restrict__ counts) {
     __shared__ double s_E[SC_MODELS][9];
@@ -1369,17 +1344,6 @@ int epv_essential_launch(epivo_ctx* ctx, const EssentialPlan& p) {
         ess_round_kernel<<<g_pairs, ES_THREADS, pts_smem, ctx->stream>>>(a, r, R[r], r == nr - 1 ? 1 : 0, pts_smem > 0);
         EPV_LAUNCHED(ctx);
     }
-#ifdef EPV_ESS_DEBUG
-    {   // debug build only: running pairs, real roots and slow-path hypotheses per round
-        int32_t ctl[ES_MAX_ROUNDS + 1], ni[ES_MAX_ROUNDS], ns[ES_MAX_ROUNDS];
-        cudaStreamSynchronize(ctx->stream);
-        cudaMemcpy(ctl, a.w.ctl, sizeof(ctl), cudaMemcpyDeviceToHost);
-        cudaMemcpy(ni, a.w.nitems, sizeof(ni), cudaMemcpyDeviceToHost);
-        cudaMemcpy(ns, a.w.nslow, sizeof(ns), cudaMemcpyDeviceToHost);
-        for (int r = 0; r < nr; ++r)
-            fprintf(stderr, "ess round %d: R %d pairs %d roots %d slow %d\n", r, R[r], ctl[r], ni[r], ns[r]);
-    }
-#endif
     return EPIVO_OK;
 }
 

@@ -191,11 +191,8 @@ __device__ __forceinline__ void pmul(const double (&a)[NA + 1], const double (&b
 // stall its warp.
 // The relative update of a sweep is tracked as a fraction (numerator, denominator) compared by
 // cross-multiplication, so a sweep costs one division per root, not two.
-#ifndef EPV_DK_FAST_SWEEPS
-#define EPV_DK_FAST_SWEEPS 32
-#endif
-constexpr int DK_FAST_SWEEPS = EPV_DK_FAST_SWEEPS;   // sweeps the fast path spends before handing a hypothesis over
-constexpr int DK_STATE = 21;                          // doubles saved for the slow pass: re[10], im[10], prev2
+constexpr int DK_FAST_SWEEPS = 32;   // sweeps the fast path spends before handing a hypothesis over
+constexpr int DK_STATE = 21;         // doubles saved for the slow pass: re[10], im[10], prev2
 
 // Sweeps [first, last) of the iteration; first == 0 sets the start values, otherwise re / im / prev2 continue a
 // previous call.  Returns true when the iteration is settled (converged, on the noise floor, or 300 sweeps done).
@@ -520,7 +517,7 @@ __device__ __forceinline__ void build_B_row(const double* rec, size_t rs, int j,
 // state (DK_STATE doubles, stride ss): written by the fast path when it returns -1, read by the slow pass.
 template <bool SLOW>
 __device__ __forceinline__ int stage_b1(const double* rec, size_t rs, double (&zs)[10], double* state = nullptr,
-                                        size_t ss = 1, double* dbg = nullptr) {
+                                        size_t ss = 1) {
     if (!(rec[36 * rs] == rec[36 * rs])) return 0;            // stage A flagged a singular system
     double B[3][3][5];
 #pragma unroll
@@ -597,12 +594,6 @@ __device__ __forceinline__ int stage_b1(const double* rec, size_t rs, double (&z
         for (int i = 0; i < 10; ++i) { re[i] = state[i * ss]; im[i] = state[(10 + i) * ss]; }
         dk_sweeps<10>(c, re, im, prev2, DK_FAST_SWEEPS, 300);
     }
-#ifdef EPV_ESS_DEBUG
-    if (dbg) {
-        for (int i = 0; i < 11; ++i) dbg[i] = c[i];
-        for (int i = 0; i < 10; ++i) { dbg[11 + i] = re[i]; dbg[21 + i] = im[i]; }
-    }
-#endif
     int count = 0;
 #pragma unroll
     for (int i = 0; i < 10; ++i) {                           // unrolled: re/im stay in registers

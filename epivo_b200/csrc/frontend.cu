@@ -372,10 +372,8 @@ __device__ __forceinline__ void lk_diff_seg(const uint8_t* __restrict__ J, int r
 }
 
 // one warp per point: all pyramid levels, all iterations
-#ifndef EPV_LK_MINBLOCKS
-#define EPV_LK_MINBLOCKS 5
-#endif
-__global__ void __launch_bounds__(128, EPV_LK_MINBLOCKS) lk_kernel(const uint8_t* __restrict__ pyr, const short2* __restrict__ dpyr, LkGeom g,
+constexpr int LK_MINBLOCKS = 5;
+__global__ void __launch_bounds__(128, LK_MINBLOCKS) lk_kernel(const uint8_t* __restrict__ pyr, const short2* __restrict__ dpyr, LkGeom g,
                                                  const float* __restrict__ pts, const int32_t* __restrict__ counts,
                                                  int max_pts, int max_count, double eps2, float min_eig,
                                                  float* __restrict__ next_pts, uint8_t* __restrict__ status,

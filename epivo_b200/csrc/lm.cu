@@ -15,9 +15,6 @@
 // Reference quirks kept on purpose: the Jacobian's Huber branch switches on e'e <= delta
 // while res switches on e'e/2 > delta (sqrt(2) mismatch at delta = 1e-5); reverse reps
 // differentiate a LEFT perturbation of the zeta although the update is right-multiplied.
-#include <stdlib.h>
-#include <string.h>
-
 #include <cooperative_groups.h>
 
 #include "common.cuh"
@@ -27,7 +24,7 @@ namespace cg = cooperative_groups;
 
 namespace {
 
-// The window kernel is instantiated for three CTA shapes <threads, points per Jacobian tile>; the launcher picks
+// The window kernel is instantiated for six CTA shapes <threads, points per Jacobian tile, cluster>; the launcher picks
 // one by problem size (measured on B200: small windows want many small CTAs, large ones wider CTAs).
 // Chain length: the reference's bound is rep_max = 128 (jac_Rt_gen_.cpp:18, the size of its memo array); its drivers
 // and demo use 4..10 zetas.  Here a window lives in shared memory -- chain memo and inverses 2 nz^2 x 96 B, H | b
@@ -471,15 +468,8 @@ __global__ void __launch_bounds__(LM_THREADS) lm_kernel(LmArgs a) {
     }
     __syncthreads();
 
-#ifdef EPV_LM_PROFILE
-    long long tp_[5] = {0, 0, 0, 0, 0}, tp0_ = clock64();
-#define LM_TICK(i) do { long long n_ = clock64(); tp_[i] += n_ - tp0_; tp0_ = n_; } while (0)
-#else
-#define LM_TICK(i) do { } while (0)
-#endif
     for (int iter = 0; iter < p.max_iters; ++iter) {
         if (tid == 0) s_iters = iter + 1;
-        LM_TICK(4);
         // ---- chain memo + inverses                                              [:328-335]
         for (int j = tid; j < nz; j += LM_THREADS) {
             Rt acc = sT[j];
@@ -498,7 +488,6 @@ __global__ void __launch_bounds__(LM_THREADS) lm_kernel(LmArgs a) {
             sRep[j] = (z0 <= z1) ? sMem[z0 * nz + z1] : sInv[z1 * nz + z0];
         }
         __syncthreads();
-        LM_TICK(0);
         // ---- residuals, Jacobian tiles, H = J'J, b = J'r
         double rsq = 0.0;
         int tile_id = 0;                            // running tile counter over all reps: tile t belongs to rank t % CL
@@ -611,7 +600,6 @@ __global__ void __launch_bounds__(LM_THREADS) lm_kernel(LmArgs a) {
                 __syncthreads();
             }
         }
-        LM_TICK(1);
         if (CL > 1) {                               // cluster reduction of the partial H | b and of |r0|^2
             rsq = lm_warp_sum(rsq);
             if ((tid & 31) == 0) sRed[tid >> 5] = rsq;
@@ -684,7 +672,6 @@ __global__ void __launch_bounds__(LM_THREADS) lm_kernel(LmArgs a) {
             }
         }
         __syncthreads();
-        LM_TICK(2);
         if (s_stop) break;
         // ---- candidate update T' = T exp(delta_k)                                  [:416-422]
         for (int k = tid; k < nz; k += LM_THREADS) {
@@ -750,18 +737,12 @@ __global__ void __launch_bounds__(LM_THREADS) lm_kernel(LmArgs a) {
             for (int k = tid; k < nz; k += LM_THREADS) sT[k] = sTn[k];
         }
         __syncthreads();
-        LM_TICK(3);
     }
     __syncthreads();
     if (CL > 1) {
         cg::this_cluster().sync();                  // no CTA may exit while a peer can still read its shared memory
         if (crank != 0) return;                     // rank 0 reports (every rank holds the same result)
     }
-#ifdef EPV_LM_PROFILE
-    if (tid == 0 && prob == 0)
-        printf("lm_kernel<%d,%d> phases (clocks): memo %lld  jac+gram %lld  solve %lld  candidate %lld  other %lld\n", LM_THREADS,
-               LM_TP, tp_[0], tp_[1], tp_[2], tp_[3], tp_[4]);
-#endif
     for (int k = tid; k < nz; k += LM_THREADS) {
         for (int i = 0; i < 3; ++i) {
             for (int j = 0; j < 3; ++j) gT[k * 16 + i * 4 + j] = sT[k].R[i * 3 + j];
@@ -781,21 +762,13 @@ __global__ void __launch_bounds__(LM_THREADS) lm_kernel(LmArgs a) {
 // One WARP per problem, everything in registers: each lane owns up to two correspondences,
 // the 6x6 normal equations are reduced with warp shuffles and solved redundantly by every lane,
 // so the 30 dependent iterations need no shared memory and no block barrier.
-#ifndef EPV_LMP_WARPS
-#define EPV_LMP_WARPS 4
-#endif
-#ifndef EPV_LMP_MINBLOCKS
-#define EPV_LMP_MINBLOCKS 1
-#endif
-constexpr int LMP_WARPS = EPV_LMP_WARPS;
+constexpr int LMP_WARPS = 4;
+constexpr int LMP_MINBLOCKS = 1;
 
 // lanes per problem: 32 = one warp per problem (two correspondences per lane); 16 / 8 pack two /
 // four problems into a warp (four / eight correspondences per lane), trading per-problem latency
 // for fewer, fuller warps -- the 30 dependent iterations make this kernel latency bound.
-#ifndef EPV_LM_LPP
-#define EPV_LM_LPP 8
-#endif
-constexpr int LM_LPP = EPV_LM_LPP;
+constexpr int LM_LPP = 8;
 constexpr int LM_PPL = 64 / LM_LPP;                 // correspondences per lane (N <= 64)
 
 __device__ __forceinline__ double group_sum_d(double v) {
@@ -804,7 +777,7 @@ __device__ __forceinline__ double group_sum_d(double v) {
     return v;
 }
 
-__global__ void __launch_bounds__(LMP_WARPS * 32, EPV_LMP_MINBLOCKS) lm_pair_kernel(LmPlan p) {
+__global__ void __launch_bounds__(LMP_WARPS * 32, LMP_MINBLOCKS) lm_pair_kernel(LmPlan p) {
     const int gl = threadIdx.x & (LM_LPP - 1);                                  // lane within the problem's group
     const int prob_raw = (blockIdx.x * LMP_WARPS * 32 + threadIdx.x) / LM_LPP;
     const bool exists = prob_raw < p.B;
@@ -1036,22 +1009,10 @@ int epv_lm_launch(epivo_ctx* ctx, const LmPlan& p) {
     // long chains: only the smallest tile leaves room for H | b and the memo
     if (lm_smem_doubles(p.n_zeta, p.n_rep, a.D, 128, 64, 1) * sizeof(double) > LM_SMEM_LIMIT)
         return lm_launch_shape<64, 32>(ctx, a);
-    // Tuning override "<threads>x<tile points>[x<cluster>]" (tools/lm_windows.py, tests).  NOTE: the shapes differ in
-    // summation order (tile boundaries, cluster partials), so the last bits of H | b -- and, on a converged plateau,
-    // the accept / reject sequence -- depend on the shape, which the launcher otherwise derives from the batch size:
-    // the same window can take a different (equally valid) trajectory in a 504-window batch and in a 63-window shard.
-    // tests/test_gpu_lm_ref.py holds every shape to the reference's result within north_star's tolerance.
-    if (const char* e = getenv("EPIVO_LM_SHAPE")) {
-        if (!strcmp(e, "384x128x2")) return lm_launch_shape<384, 128, 2>(ctx, a);
-        if (!strcmp(e, "256x128x2")) return lm_launch_shape<256, 128, 2>(ctx, a);
-        if (!strcmp(e, "256x64x4")) return lm_launch_shape<256, 64, 4>(ctx, a);
-        if (!strcmp(e, "384x64x4")) return lm_launch_shape<384, 64, 4>(ctx, a);
-        if (!strcmp(e, "512x128")) return lm_launch_shape<512, 128>(ctx, a);
-        if (!strcmp(e, "384x128")) return lm_launch_shape<384, 128>(ctx, a);
-        if (!strcmp(e, "256x128")) return lm_launch_shape<256, 128>(ctx, a);
-        if (!strcmp(e, "192x96")) return lm_launch_shape<192, 96>(ctx, a);
-        if (!strcmp(e, "128x64")) return lm_launch_shape<128, 64>(ctx, a);
-    }
+    // The shapes differ in summation order (tile boundaries, cluster partials), so the last bits of H | b -- and, on a
+    // converged plateau, the accept / reject sequence -- depend on the shape, which follows from the batch size: the
+    // same window can take a different (equally valid) trajectory in a 504-window batch and in a 63-window shard.
+    // tests/test_gpu_lm_ref.py holds every shape below to the reference's result within north_star's tolerance.
     if (p.N <= 32) return lm_launch_shape<64, 32>(ctx, a);          // e.g. the shipped kitti_ba shape: 9 reps x 32 points
     // few large windows (a multi-GPU shard of cfg5: 63 windows per GPU): every CTA has an SM to itself, so the
     // wider CTA wins (63 cfg5 windows: 11.3 ms against 14.0 ms); with several CTAs per SM the narrower one does

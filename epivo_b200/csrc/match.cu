@@ -25,25 +25,11 @@
 
 namespace {
 
-#ifndef EPV_MT_THREADS
-#define EPV_MT_THREADS 128
-#endif
-#ifndef EPV_MT_RQ
-#define EPV_MT_RQ 8
-#endif
-#ifndef EPV_MT_MINBLOCKS
-#define EPV_MT_MINBLOCKS 4
-#endif
-constexpr int MT_THREADS = EPV_MT_THREADS;
-constexpr int MT_RQ = EPV_MT_RQ;
-#ifndef EPV_MT_TILE
-#define EPV_MT_TILE 128
-#endif
-#ifndef EPV_MT_UNROLL
-#define EPV_MT_UNROLL 1
-#endif
-constexpr int MT_TILE = EPV_MT_TILE;
-constexpr int MT_UNROLL = EPV_MT_UNROLL;
+constexpr int MT_THREADS = 128;
+constexpr int MT_RQ = 8;
+constexpr int MT_MINBLOCKS = 4;
+constexpr int MT_TILE = 128;
+constexpr int MT_UNROLL = 1;
 
 __device__ __forceinline__ uint32_t smem_u32(const void* p) {
     return static_cast<uint32_t>(__cvta_generic_to_shared(p));
@@ -128,7 +114,7 @@ __device__ __forceinline__ uint32_t desc_dist(const uint32_t (&q)[WORDS], const 
 // RQ = query rows per thread: 8 (a CTA covers 1024 query rows) or 6 (768), whichever wastes fewer row slots for the
 // given set size -- 1500 EuRoC keypoints are two CTAs either way, but 2 x 768 instead of 2 x 1024 slots (mt_pick_rq).
 template <int WORDS, int RQ, bool NORM2, bool TOP2, bool COUNTS>
-__global__ void __launch_bounds__(MT_THREADS, WORDS <= 8 ? EPV_MT_MINBLOCKS : 1)   // 64-byte descriptors need the registers
+__global__ void __launch_bounds__(MT_THREADS, WORDS <= 8 ? MT_MINBLOCKS : 1)   // 64-byte descriptors need the registers
 match_tile_kernel(const uint32_t* __restrict__ desc, int64_t q0, int64_t qs, int64_t t0, int64_t ts, int nq,
                   int nt, uint32_t* __restrict__ rowkey, uint32_t* __restrict__ rowkey2,
                   uint32_t* __restrict__ colkey, int stride, int tiles_per_split, int64_t part_stride,

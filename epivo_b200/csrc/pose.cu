@@ -17,13 +17,8 @@
 
 namespace {
 
-#ifndef EPV_PS_THREADS
-#define EPV_PS_THREADS 128
-#endif
-#ifndef EPV_PS_MINBLOCKS
-#define EPV_PS_MINBLOCKS 4
-#endif
-constexpr int PS_THREADS = EPV_PS_THREADS;
+constexpr int PS_THREADS = 128;
+constexpr int PS_MINBLOCKS = 4;
 
 // Cyclic Jacobi eigen-decomposition of a symmetric NxN matrix (N = 3, 4): A -> diag, V = eigenvectors (columns)
 template <int N>
@@ -239,7 +234,7 @@ __device__ __forceinline__ unsigned triangulate_good2(const double* R, const dou
     return (gp ? 1u : 0u) | (gn ? 2u : 0u);
 }
 
-__global__ void __launch_bounds__(PS_THREADS, EPV_PS_MINBLOCKS) pose_kernel(PosePlan p) {
+__global__ void __launch_bounds__(PS_THREADS, PS_MINBLOCKS) pose_kernel(PosePlan p) {
     __shared__ double s_R[2][9];
     __shared__ double s_t[3];
     __shared__ int s_cnt[4];

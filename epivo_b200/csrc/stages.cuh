@@ -67,8 +67,8 @@ struct LmPlan {
     int single_pair;         // caller asserts reps == {(0,0)}: warp-per-problem kernel when n_zeta == 1, N <= 64
 };
 int epv_lm_launch(epivo_ctx* ctx, const LmPlan& p);
-// epv_lm_launch's refusals for a problem with N <= 32 points per rep (the shape it then picks, 64 x 32, unless
-// EPIVO_LM_SHAPE overrides it), without launching: for callers that check everything before their first launch
+// epv_lm_launch's refusals for a problem with N <= 32 points per rep (the shape it then picks, 64 x 32), without
+// launching: for callers that check everything before their first launch
 int epv_lm_check_n32(epivo_ctx* ctx, int n_zeta, int n_rep);
 
 // ---- cloud.cu (N2: pose chain + per-inlier depth / point cloud, kitti_E.cpp:203-254) ------

@@ -32,18 +32,29 @@ def test_gpu_lm_equals_reference_build(ctx, name, tag):
         assert np.array_equal(T, c["T0s"])                    # "delta has Nan" before any update (:407)
 
 
-@pytest.mark.parametrize("shape", ["384x128x2", "256x64x4", "192x96", "128x64"])
-def test_gpu_lm_cfg5_every_kernel_shape_equals_reference_build(ctx, shape, monkeypatch):
-    """The window kernel's CTA / cluster shapes differ in summation order only: each one must meet the
-    reference on BASELINE config 5 (and on the demo chain) at both Huber settings."""
+# epv_lm_launch picks the shape of a window with N >= 96 points per rep from the batch size B against the SM count
+# (the value epivo_create reads): a cluster of 4 CTAs while 4 B <= SMs, of 2 while 2 B <= SMs, one 384-thread CTA
+# while B <= SMs, else a 192-thread CTA
+WIDE_SHAPE_BATCH = {"384x64x4": lambda sms: 1, "384x128x2": lambda sms: sms // 2, "384x128": lambda sms: sms,
+                    "192x96": lambda sms: sms + 1}
+
+
+@pytest.mark.parametrize("shape", list(WIDE_SHAPE_BATCH))
+def test_gpu_lm_cfg5_on_every_launched_shape_equals_reference_build(ctx, shape):
+    """The window kernel's shapes differ in summation order only: B copies of BASELINE config 5 in one batch, with B
+    chosen so that the launcher picks `shape`, must meet the reference at both Huber settings, and every copy must
+    equal the first bit for bit (one shape, one summation order).  The demo chain (N = 15) runs the 64 x 32 shape in
+    test_gpu_lm_equals_reference_build."""
+    import torch
     from epivo_b200 import api
-    monkeypatch.setenv("EPIVO_LM_SHAPE", shape)
-    for name in ("cfg5_51", "demo_refgen_3"):
-        c = case(name)
-        for tag in ("ref", "d1"):
-            T, info = api.Levenberg_Marquardt(c["n_zeta"], EPSILON, c["reps"], c["wreps"], LAMBDA0, c["T0s"], c["pr"],
-                                              c["p_r"], huber_delta=DELTAS[tag], ctx=ctx)
-            check(name, tag, T, info["r_norm"], info["lambda"], info["H_norm"])
+    B = WIDE_SHAPE_BATCH[shape](torch.cuda.get_device_properties(0).multi_processor_count)
+    c = case("cfg5_51")
+    for tag in ("ref", "d1"):
+        Tb, res, its = api.Levenberg_Marquardt_batch(c["n_zeta"], EPSILON, c["reps"], c["wreps"], LAMBDA0,
+                                                     np.stack([c["T0s"]] * B), np.stack([c["pr"]] * B),
+                                                     np.stack([c["p_r"]] * B), huber_delta=DELTAS[tag], ctx=ctx)
+        check("cfg5_51", tag, Tb[0], res[0][1], res[0][2], res[0][0])
+        assert (Tb == Tb[0]).all() and (res == res[0]).all() and (its == its[0]).all()
 
 
 def test_gpu_lm_batch_of_kitti_e_pairs_equals_reference_build(ctx):

@@ -18,11 +18,6 @@ pytestmark = pytest.mark.gpu
 FALLBACK_T = np.array([0.1, 0.1, -0.9])
 
 
-@pytest.fixture(autouse=True)
-def _default_lm_shape(monkeypatch):
-    monkeypatch.delenv("EPIVO_LM_SHAPE", raising=False)
-
-
 def window_ws(ws):
     """main(): kitti_ba.cpp:1131-1144."""
     w = []

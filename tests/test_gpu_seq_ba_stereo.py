@@ -17,11 +17,6 @@ from test_gpu_seq_ba import _code, _kept, _params, _unfused, window_ws
 pytestmark = pytest.mark.gpu
 
 
-@pytest.fixture(autouse=True)
-def _default_lm_shape(monkeypatch):
-    monkeypatch.delenv("EPIVO_LM_SHAPE", raising=False)
-
-
 def _stereo_pairs(window, stride, F):
     """The node pair list of the stereo driver: every key its windows read, chain pairs (2f+1, 2f+2) included."""
     return ba.window_pairs(ba.expand_stereo_window(window), 2 * stride, 2 * F)

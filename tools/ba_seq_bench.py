@@ -102,7 +102,6 @@ def main():
     stereo = len(args) < len(sys.argv) - 1
     F = int(args[0]) if len(args) > 0 else 1009
     reps = int(args[1]) if len(args) > 1 else 10
-    os.environ.pop("EPIVO_LM_SHAPE", None)
     if stereo:
         seq = synth.make_sequence(n_frames=2 * F, n=2000)
         pairs = ba.window_pairs(ba.expand_stereo_window(WINDOW), 2 * STRIDE, 2 * F)

@@ -20,7 +20,7 @@ for _ in range(5):
 res = pipe.download(0, seq.n_pairs)
 it = res["ransac_iters"]
 names = ["total", "match", "presolve", "essential", "pose", "lm", "finish", "match_kernel"]
-print(os.environ.get("EPIVO_VARIANT", "product"), {k: round(float(acc[i] / 5), 3) for i, k in enumerate(names)})
+print({k: round(float(acc[i] / 5), 3) for i, k in enumerate(names)})
 import signal; signal.signal(signal.SIGPIPE, signal.SIG_DFL)
 print("iters: mean %.2f  <=8 %.3f  <=12 %.3f  <=16 %.3f  <=24 %.3f  <=32 %.3f  max %d" %
       (it.mean(), (it <= 8).mean(), (it <= 12).mean(), (it <= 16).mean(), (it <= 24).mean(), (it <= 32).mean(), it.max()))
